@@ -425,6 +425,31 @@ class Runner:
             self.reducer.unbind()
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(run, out_dir):
+    """Writes what the last step of the timed loop handed its caller: the loss and the gradient of every parameter that
+    receives one, as float32 ``DIR/loss.npy`` and ``DIR/grad.<parameter name>.npy``.  Inputs and weights are seeded, so
+    two builds run with the same arguments can be compared array for array.  Above DUMP_LIMIT_BYTES in all, every array
+    is replaced by the same fraction of its elements, flattened, at indices drawn from a fixed seed (the same arguments
+    give the same indices, so two builds' samples stay comparable).  Returns the number of bytes written."""
+    torch.cuda.synchronize()
+    arrays = {"loss": run.loss_buf.reshape(-1)[:1]}
+    arrays.update({f"grad.{k}": p.grad for k, p in run.model.named_parameters() if p.grad is not None})
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        frac = (DUMP_LIMIT_BYTES - 4 * len(arrays)) / total        # the max(1, ...) below adds at most one element each
+        rng = np.random.default_rng(0)
+        arrays = {k: v.reshape(-1)[np.sort(rng.choice(v.size, max(1, int(v.size * frac)), replace=False))]
+                  for k, v in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), v)
+    return sum(v.nbytes for v in arrays.values())
+
+
 def _short_line(r, value, ms_step, extra=None):
     fwd_f, tot_f, _ = flops_per_sample(r.n, r.kind, r.ks, blocks=r.blocks)
     d = {"workload": f"{r.desc} batch={r.B}/GPU x {r.world} GPU", "precision": r.precision, "value": value,
@@ -453,7 +478,14 @@ def main():
     ap.add_argument("--no-graph", action="store_true", help="launch the step eagerly instead of replaying a CUDA graph")
     ap.add_argument("--max-seconds", type=int, default=int(os.environ.get("STGCN_BENCH_MAX_SECONDS", "900")),
                     help="watchdog: dump all Python stacks to stderr and exit 124 if the run has not finished by then")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the loss and parameter gradients of the last timed step as "
+                         "float32 DIR/<name>.npy (seeded inputs: two builds can be compared output for output)")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -472,7 +504,7 @@ def main():
         if rank != 0:
             return
         cpu_b = min(B, 32 if a.workload != "syn2048" else 2)       # ~1 GFLOP of conv/bmm per sample-step at N=2048
-        r = cpu_reference_run(a.workload, cpu_b, max(steps, 10), warmup, a.droprate)
+        r = cpu_reference_run(a.workload, cpu_b, steps, warmup, a.droprate)
         what = "the unmodified reference (baseline/_ref)" if r["kind"] == "reference" else \
             "oracle port of the reference step (same ATen ops)"
         sample = (f"median of {r['steps']} steps of B={cpu_b} (a bounded sample of the B={B} workload: "
@@ -522,6 +554,9 @@ def main():
     ms_total = run.timed(run.step, steps)
     launches = (L.launch_count() - n0) if run.graphed is None else run.launches_per_step * steps
     value = B * world * steps / (ms_total / 1e3)
+    if a.dump_outputs and rank == 0:            # before the end-to-end leg overwrites the loss and gradients
+        nbytes = dump_outputs(run, a.dump_outputs)
+        print(f"[bench] last timed step's loss and gradients: {nbytes} bytes under {a.dump_outputs}", file=sys.stderr)
 
     for i in range(2):
         run.e2e_step(i)

@@ -7,8 +7,8 @@ numpy restatements of
   * the reference's own Lion optimizer (script/opt.py:34-76),
   * data_transform, the window construction (script/dataloader.py:32-48).
 Pinned by tests/test_train_oracle.py: AdamW against the installed torch.optim.AdamW, Lion and data_transform against
-vectors generated from the UNMODIFIED reference by tests/golden/make_train_golden.py (tests/golden/train_*.npz), and live
-against the reference when /root/reference is mounted."""
+vectors generated from the UNMODIFIED reference by tests/golden/make_train_golden.py (tests/golden/train_*.npz) and
+tests/golden/make_ref_golden.py (tests/golden/ref_windows_small.npz)."""
 from __future__ import annotations
 
 import numpy as np

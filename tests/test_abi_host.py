@@ -2,18 +2,16 @@
 the ctypes mirror has the header's struct layouts, size queries and error reporting work without a GPU, and the
 module API keeps the reference's state_dict contract."""
 import ctypes as C
+import json
 import os
 import re
 import subprocess
-import sys
 import tempfile
-import types
-import importlib.util
 
 import pytest
 import torch
 
-from conftest import ROOT, GoldenCase, golden_case_names
+from conftest import GOLDEN, ROOT, GoldenCase, golden_case_names
 
 HEADER = os.path.join(ROOT, "include", "stgcn_b200.h")
 
@@ -115,38 +113,26 @@ def test_no_cpu_fallback():
         m(g.x)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/model"), reason="reference not mounted")
-def test_reference_models_py_loads_our_layers_unchanged():
-    """The drop-in claim: the reference's own model/models.py, executed unmodified with `model.layers`
-    resolving to stgcn_b200.layers, builds a network with the reference's state_dict."""
+def test_reference_models_py_calls_build_our_layers():
+    """The drop-in claim: the layer constructor calls the reference's own model/models.py makes (recorded with their
+    arguments and the submodule each result is stored under, tests/golden/make_ref_golden.py), replayed on
+    stgcn_b200.layers, build a network with the reference's state_dict."""
     import stgcn_b200.layers as ours
-    saved = {k: sys.modules.get(k) for k in ("model", "model.layers", "model.models")}
-    try:
-        pkg = types.ModuleType("model")
-        pkg.__path__ = []
-        pkg.layers = ours
-        sys.modules["model"] = pkg
-        sys.modules["model.layers"] = ours
-        spec = importlib.util.spec_from_file_location("model.models", "/root/reference/model/models.py")
-        ref_models = importlib.util.module_from_spec(spec)
-        spec.loader.exec_module(ref_models)
-        from types import SimpleNamespace
-        for name in ("pemsd7m_cheb3_glu", "tiny_gcn_glu"):
-            g = GoldenCase(name)
-            c = g.cfg
-            args = SimpleNamespace(Kt=c["Kt"], Ks=c["Ks"], act_func=c["act"], graph_conv_type=c["kind"], gso=g.gso,
-                                   enable_bias=c["bias"], droprate=0.5, n_his=c["n_his"])
-            cls = ref_models.STGCNChebGraphConv if c["kind"] == "cheb_graph_conv" else ref_models.STGCNGraphConv
-            m = cls(args, c["blocks"], c["n"])
-            assert type(m.st_blocks[0]).__module__ == "stgcn_b200.layers"
-            assert list(m.state_dict().keys()) == list(g.params.keys())
-            m.load_state_dict(g.params, strict=True)
-    finally:
-        for k, v in saved.items():
-            if v is None:
-                sys.modules.pop(k, None)
+    with open(os.path.join(GOLDEN, "ref_models_calls.json")) as f:
+        calls = json.load(f)
+    for name in ("pemsd7m_cheb3_glu", "tiny_gcn_glu"):
+        g = GoldenCase(name)
+        m = torch.nn.Module()
+        for e in calls[name]:
+            parent, _, attr = e["path"].rpartition(".")
+            if "container" in e:
+                child = getattr(torch.nn, e["container"])()
             else:
-                sys.modules[k] = v
+                child = getattr(ours, e["layer"])(*[g.gso if a == "gso" else a for a in e["args"]])
+                assert type(child).__module__ == "stgcn_b200.layers"
+            m.get_submodule(parent).add_module(attr, child)
+        assert list(m.state_dict().keys()) == list(g.params.keys())
+        m.load_state_dict(g.params, strict=True)
 
 
 def _sizes_in_subprocess(env_extra):

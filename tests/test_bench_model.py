@@ -48,6 +48,34 @@ def test_kernel_work_model_and_traffic_table():
     assert bench._ncu_traffic("st0.tc2.fwd:umma_tap_kernel<EPI_GATE>", "metrla", 512, "bf16") is None
 
 
+def test_dump_outputs_full_and_sampled(tmp_path, monkeypatch):
+    """--dump-outputs: the loss and every existing gradient as float32 .npy; over the size limit, a seeded sample of
+    every array that is the same from run to run and stays within the limit."""
+    import types
+    import numpy as np
+    import torch
+    monkeypatch.setattr(torch.cuda, "synchronize", lambda *a: None)
+    model = torch.nn.Sequential(torch.nn.Linear(300, 200), torch.nn.Linear(200, 3), torch.nn.Linear(3, 3))
+    for p in list(model.parameters())[:4]:
+        p.grad = torch.randn_like(p)
+    run = types.SimpleNamespace(model=model, loss_buf=torch.tensor([0.25]))
+    names = {"loss.npy", "grad.0.weight.npy", "grad.0.bias.npy", "grad.1.weight.npy", "grad.1.bias.npy"}
+    full = bench.dump_outputs(run, str(tmp_path / "full"))
+    assert set(os.listdir(tmp_path / "full")) == names
+    assert full == 4 * (1 + 300 * 200 + 200 + 200 * 3 + 3)
+    w = np.load(tmp_path / "full" / "grad.0.weight.npy")
+    assert w.dtype == np.float32 and np.array_equal(w, model[0].weight.grad.numpy())
+    assert np.load(tmp_path / "full" / "loss.npy").tolist() == [0.25]
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", full // 10)
+    for d in ("a", "b"):
+        assert bench.dump_outputs(run, str(tmp_path / d)) <= full // 10
+    for n in names:
+        a, b = np.load(tmp_path / "a" / n), np.load(tmp_path / "b" / n)
+        assert a.dtype == np.float32 and a.ndim == 1 and np.array_equal(a, b), n
+    sample = np.load(tmp_path / "a" / "grad.0.weight.npy")
+    assert 0 < sample.size < w.size and np.isin(sample, w).all()
+
+
 def test_synthetic_sweep_workload_model():
     """BASELINE configs[4] (N=2048, Ks=5, 64 graph-conv channels): FLOPs / bytes of SURVEY.md §8(d) with the workload's
     own block table, and the seeded operator has spectral norm 1 (checked at a small size; same constructor)."""

@@ -1,11 +1,12 @@
 """Pins oracle/stgcn_oracle.py against the reference-generated golden vectors (CPU)."""
+import json
 import os
-import sys
 
+import numpy as np
 import pytest
 import torch
 
-from conftest import GoldenCase, golden_case_names, rel_l2
+from conftest import GOLDEN, GoldenCase, golden_case_names, rel_l2
 from oracle import stgcn_oracle as O
 
 TOL = 2e-5   # fp32 vs fp32 of the same math, different op fusion/order
@@ -63,24 +64,16 @@ def test_oracle_errors_match_reference_behaviour():
         O.cheb_graph_conv(x, torch.eye(3), torch.zeros(0, 2, 2), None)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/model"), reason="reference not mounted")
-def test_oracle_live_against_reference():
-    """When the reference is mounted (build container), compare live on a fresh seed."""
-    sys.path.insert(0, "/root/reference")
-    try:
-        from model import models as ref_models
-    finally:
-        sys.path.pop(0)
-    from types import SimpleNamespace
-    torch.manual_seed(123)
-    n = 23
-    gso = O.synthetic_gso(n, seed=5)
-    blocks = [[1], [16, 8, 16], [16, 8, 16], [32, 32], [1]]
-    for kind, cls in (("cheb_graph_conv", ref_models.STGCNChebGraphConv), ("graph_conv", ref_models.STGCNGraphConv)):
-        args = SimpleNamespace(Kt=3, Ks=3, act_func="glu", graph_conv_type=kind, gso=gso, enable_bias=True,
-                               droprate=0.0, n_his=12)
-        m = cls(args, blocks, n)
-        x = torch.randn(4, 1, 12, n)
-        ref = m(x)
-        got = O.stgcn_forward(x, dict(m.state_dict()), gso, blocks=blocks, kt=3, n_his=12, act="glu", kind=kind)
-        assert rel_l2(got, ref) < TOL
+def test_oracle_matches_reference_forward_n23():
+    """The reference's forward of both model classes on default-initialised weights of a fresh seed
+    (tests/golden/make_ref_golden.py, ref_forward_n23.npz)."""
+    z = np.load(os.path.join(GOLDEN, "ref_forward_n23.npz"))
+    gso = torch.from_numpy(z["gso"])
+    assert torch.equal(gso, O.synthetic_gso(23, seed=5))
+    blocks = json.loads(str(z["blocks"]))
+    for kind in ("cheb_graph_conv", "graph_conv"):
+        params = {k[len(kind) + 3:]: torch.from_numpy(z[k]) for k in z.files if k.startswith(f"{kind}/p:")}
+        x, ref = torch.from_numpy(z[f"{kind}/x"]), torch.from_numpy(z[f"{kind}/out"])
+        got = O.stgcn_forward(x, params, gso, blocks=blocks, kt=3, n_his=12, act="glu", kind=kind)
+        assert tuple(got.shape) == tuple(ref.shape)
+        assert rel_l2(got, ref) < TOL, kind
