@@ -212,6 +212,29 @@ int stgcn_outblock_bwd(const stgcn_outblock_desc*, const void* x, const void* sa
                        const stgcn_outblock_params*, const stgcn_outblock_grads*, void* dx,
                        void* workspace, size_t workspace_bytes, uint64_t dropout_seed, void* stream);
 
+/* ---- inference: the block forwards with no backward state ------------------------------ */
+/* STConvBlock / OutputBlock forward under torch.no_grad() (the model.eval() passes of val() / test(), main.py:184-203):
+ * same desc / params / x / y and the same result, bit for bit, as *_fwd -- including training / p_drop / dropout_seed and
+ * the step counter of stgcn_set_dropout_step -- but nothing a backward would read is kept: there is no `saved` buffer,
+ * every intermediate lives in the workspace only while it is needed, and the kernels skip the stores of the gate
+ * pre-activations and Chebyshev planes where they can.  Same statuses and messages as *_sizes / *_fwd.               */
+int stgcn_stblock_infer_sizes(const stgcn_stblock_desc*, size_t* workspace_bytes);
+int stgcn_stblock_infer(const stgcn_stblock_desc*, const void* x, const stgcn_stblock_params*, void* y,
+                        void* workspace, size_t workspace_bytes, uint64_t dropout_seed, void* stream);
+int stgcn_outblock_infer_sizes(const stgcn_outblock_desc*, size_t* workspace_bytes);
+int stgcn_outblock_infer(const stgcn_outblock_desc*, const void* x, const stgcn_outblock_params*, void* y,
+                         void* workspace, size_t workspace_bytes, uint64_t dropout_seed, void* stream);
+/* evaluate_model / evaluate_metric (script/utility.py:90-121) of one batch, accumulated on the device.  pred, target:
+ * (B, N) fp32, normalised.  acc: device double[4], zeroed by the caller, to which this adds
+ *   acc[0] += sum (pred - target)^2                      (the MSELoss of evaluate_model, on normalised values)
+ *   acc[1] += sum |y - y_pred|,  acc[2] += sum |y - y_pred|^2,  acc[3] += sum y
+ * where y / y_pred are target / pred after StandardScaler.inverse_transform on float32 arrays: x * scale[n], then
+ * + mean[n], each rounded to float32 (pass scaler.scale_ / scaler.mean_ rounded to float32; NULL skips the step, as
+ * with_std / with_mean = False do); |d| and d^2 are float32, as numpy computes them.  Deterministic (fixed-order fp64
+ * sums, no atomics), no allocation, no host synchronisation, capturable.  N <= 16384.                                  */
+int stgcn_eval_accumulate(const float* pred, const float* target, int32_t B, int32_t N, const float* mean,
+                          const float* scale, double* acc, void* stream);
+
 /* ---- diagnostics ---------------------------------------------------------------------- */
 /* Minimal tcgen05 GEMM (bf16 operands, fp32 TMEM accumulate) exercising the operand layouts of the
  * production kernels; see csrc/umma_selftest.cuh for the modes.  Used by tests only.         */

@@ -3,7 +3,7 @@
 Importing this package never touches the GPU; the shared library is loaded on first use and there is no
 fallback if it is missing (``stgcn_b200._lib.lib()`` raises).
 """
-from . import _lib, layers, models, dist, graph, optim, data, gso, synthetic
+from . import _lib, layers, models, dist, graph, optim, data, gso, synthetic, evaluate
 from .layers import (Align, CausalConv1d, CausalConv2d, TemporalConvLayer, ChebGraphConv, GraphConv, GraphConvLayer,
                      STConvBlock, OutputBlock, set_precision, get_precision)
 from ._lib import StgcnError, launch_count

@@ -118,6 +118,11 @@ _SIGNATURES = [
     ("stgcn_outblock_fwd", C.c_int, [_P(OutblockDesc), _fp, _P(OutblockParams), _fp, _fp, _fp, _sz, C.c_uint64, _fp]),
     ("stgcn_outblock_bwd", C.c_int, [_P(OutblockDesc), _fp, _fp, _fp, _P(OutblockParams), _P(OutblockGrads), _fp,
                                      _fp, _sz, C.c_uint64, _fp]),
+    ("stgcn_stblock_infer_sizes", C.c_int, [_P(StblockDesc), _P(_sz)]),
+    ("stgcn_stblock_infer", C.c_int, [_P(StblockDesc), _fp, _P(StblockParams), _fp, _fp, _sz, C.c_uint64, _fp]),
+    ("stgcn_outblock_infer_sizes", C.c_int, [_P(OutblockDesc), _P(_sz)]),
+    ("stgcn_outblock_infer", C.c_int, [_P(OutblockDesc), _fp, _P(OutblockParams), _fp, _fp, _sz, C.c_uint64, _fp]),
+    ("stgcn_eval_accumulate", C.c_int, [_fp, _fp, C.c_int32, C.c_int32, _fp, _fp, _fp, _fp]),
     ("stgcn_umma_selftest", C.c_int, [C.c_int, _fp, _fp, _fp, C.c_int, C.c_int, C.c_int, C.c_uint32, C.c_uint32,
                                       C.c_uint32, C.c_uint32, _fp]),
     ("stgcn_debug_timeline", C.c_int, [_fp]),

@@ -153,6 +153,19 @@ inline size_t tconv_saved_elems(const stgcn_tconv_desc& d, bool q_only = false) 
   auto g = tconv_geom(d);
   return (size_t)g.rows_out * (q_only ? d.c_out : g.W);
 }
+// whether tconv_fwd's tcgen05 path serves this shape (shapes only, placeholder pointers)
+inline bool tconv_tap_served(const stgcn_tconv_desc& d, bool q_only) {
+  if (d.B <= 0) return false;
+  TconvGeom g = tconv_geom(d);
+  umma::TapProblem q{};
+  q.B = d.B; q.N = d.N; q.T_src = d.T; q.T_out = g.T_out; q.Kt = d.Kt; q.t0 = 0;
+  q.Cin = d.c_in; q.Co = g.W; q.epi = umma::EPI_GATE; q.act = d.act; q.Cout = d.c_out;
+  const bool explicit_res = !(g.folded || g.linear);
+  q.aux = explicit_res ? reinterpret_cast<const simt::bf16*>(256) : nullptr; q.C_aux = d.c_in;
+  q.aux_cols = d.c_in < d.c_out ? d.c_in : d.c_out;
+  q.q_only = q_only ? 1 : 0;
+  return umma::tap_supported(q);
+}
 // GLU "q-only" saved state (block-level callers that own both directions): the tcgen05 forward stores only the gate
 // half Q of the pre-activation; the backward gets du = dy*s, dq = dy*h*(1-s) from Q and the layer output h, which the
 // block keeps anyway.  Saves a 64-channel store + load per gated conv.  Shapes only, so forward and backward agree.
@@ -160,17 +173,28 @@ template <class T>
 inline bool tconv_qonly(const stgcn_tconv_desc& d) {
   if constexpr (std::is_same<T, simt::bf16>::value) {
     if (d.act != STGCN_ACT_GLU || d.B <= 0) return false;      // validated +5.8% (profiles/r01_ab_batch_g.md)
-    TconvGeom g = tconv_geom(d);
-    umma::TapProblem q{};
-    q.B = d.B; q.N = d.N; q.T_src = d.T; q.T_out = g.T_out; q.Kt = d.Kt; q.t0 = 0;
-    q.Cin = d.c_in; q.Co = g.W; q.epi = umma::EPI_GATE; q.act = d.act; q.Cout = d.c_out;
-    const bool explicit_res = !(g.folded || g.linear);
-    q.aux = explicit_res ? reinterpret_cast<const simt::bf16*>(256) : nullptr; q.C_aux = d.c_in;
-    q.aux_cols = d.c_in < d.c_out ? d.c_in : d.c_out;
-    q.q_only = 1;
-    return umma::tap_supported(q) && d.c_out % 8 == 0;
+    return tconv_tap_served(d, true) && d.c_out % 8 == 0;
   }
   return false;
+}
+// whether tconv_fwd may be called with z_saved == nullptr: the tcgen05 tap kernel (bf16; not for the gates that have no
+// inference instantiation, umma::tap_nz_spills) and the c_in == 1 kernel keep the pre-activations on chip; the other paths
+// write z and read it back.  Shapes only; the c_in == 1 kernel also wants y 16-byte aligned, which every arena block is.
+template <class T>
+inline bool tconv_z_optional(const stgcn_tconv_desc& d, bool q_only) {
+  const TconvGeom g = tconv_geom(d);
+  if constexpr (std::is_same<T, simt::bf16>::value) {
+    if (tconv_tap_served(d, q_only)) {
+      umma::TapProblem q{};                        // tconv_fwd's problem, placeholder pointers (in == aux, bias present)
+      const simt::bf16* ph = reinterpret_cast<const simt::bf16*>(256);
+      q.in = ph; q.bias = reinterpret_cast<const float*>(256); q.B = d.B; q.N = d.N; q.T_src = d.T; q.T_out = g.T_out;
+      q.Kt = d.Kt; q.t0 = 0; q.Cin = d.c_in; q.Co = g.W; q.epi = umma::EPI_GATE; q.act = d.act; q.Cout = d.c_out;
+      q.aux = (g.folded || g.linear) ? nullptr : ph; q.aux_dt = d.Kt - 1; q.T_aux = d.T; q.C_aux = d.c_in;
+      q.aux_cols = d.c_in < d.c_out ? d.c_in : d.c_out; q.q_only = q_only ? 1 : 0;
+      return !umma::tap_nz_spills(d.act, umma::tap_aux_epilogue(q));
+    }
+  }
+  return g.rows_out > 0 && smallc_supported<T>(d.c_in, d.c_out, g.W, d.Kt) && smallc1_supported<T>(d.c_in, d.c_out, d.Kt);
 }
 
 // z_saved: [rows_out, W] pre-activations
@@ -238,12 +262,14 @@ inline void tconv_fwd(const stgcn_tconv_desc& d, const T* x, const stgcn_tconv_p
       launch_smallc1_conv_gate_fwd(sa, c.stream);
       return;
     }
+    STGCN_CHECK(z_saved, STGCN_E_INVALID, "tconv_fwd: this path needs a pre-activation buffer");
     size_t smem = (size_t)(d.Kt * d.c_in + 1) * g.W * sizeof(float);
     long long total = g.rows_out * (d.c_out / 8);
     int blocks = (int)std::min<long long>(ceil_div(total, 256), 148 * 16);
     STGCN_LAUNCH(smallc_conv_gate_fwd_kernel<T>, blocks, 256, smem, c.stream, sa);
     return;
   }
+  STGCN_CHECK(z_saved || g.rows_out == 0, STGCN_E_INVALID, "tconv_fwd: this path needs a pre-activation buffer");
   TapArgs<T> t{};
   t.in = x; t.wt = wt; t.bias = bias; t.out = z_saved; t.rows = g.rows_out;
   t.Cin = d.c_in; t.Co = g.W; t.ntaps = d.Kt; t.ldo = g.W; t.accumulate = 0;
@@ -475,9 +501,11 @@ inline bool gconv_fused(const stgcn_gconv_desc& d) {
   return false;
 }
 
-// stack: [depth][rows, C]; stack[0] = aligned input, stack[k] = T_k(L) stack[0] (cheb) / L stack[0] (gcn)
+// stack: [depth][rows, C]; stack[0] = aligned input, stack[k] = T_k(L) stack[0] (cheb) / L stack[0] (gcn).
+// planes == false (inference, fused kernel only): stack holds plane 0 alone; planes 1.. never reach HBM.
 template <class T>
-inline void gconv_fwd(const stgcn_gconv_desc& d, const T* x, const stgcn_gconv_params& p, T* y, T* stack, Ctx c) {
+inline void gconv_fwd(const stgcn_gconv_desc& d, const T* x, const stgcn_gconv_params& p, T* y, T* stack, Ctx c,
+                      bool planes = true) {
   gconv_check(d);
   ScopedMark sm(c.ws);
   const long long rows = (long long)d.B * d.T * d.N;
@@ -492,6 +520,7 @@ inline void gconv_fwd(const stgcn_gconv_desc& d, const T* x, const stgcn_gconv_p
   const bool fused = gconv_fused<T>(d);
   if (c.dry()) return;
   STGCN_CHECK(p.w && p.gso, STGCN_E_INVALID, "gconv: missing weight or gso");
+  STGCN_CHECK(planes || fused, STGCN_E_INVALID, "gconv_fwd: only the fused kernel runs without the stack planes");
   T* x0 = stack;
   bool align_done = false, mix_done = false;
   if constexpr (std::is_same<T, simt::bf16>::value) {
@@ -523,7 +552,7 @@ inline void gconv_fwd(const stgcn_gconv_desc& d, const T* x, const stgcn_gconv_p
       umma::ChebProblem q{};
       q.N = d.N; q.G = (long long)d.B * d.T; q.depth = fdepth; q.tap_first = d.gconv == STGCN_GCONV_CHEB ? 0 : 1;
       q.n_taps = ftaps; q.relu = d.relu; q.residual = d.residual; q.a_mat = mbf; q.w = p.w; q.bias = p.b;
-      q.in = x0; q.stack = stack; q.out = y;
+      q.in = x0; q.stack = planes ? stack : nullptr; q.out = y;
       umma::launch_cheb(q, false, c.stream);
       return;
     }
@@ -929,6 +958,43 @@ inline void stblock_fwd(const stgcn_stblock_desc& d, const T* x, const stgcn_stb
   { Tag t(first ? "st0.ln.fwd" : "st1.ln.fwd"); lnorm_fwd<T>(g.ln, s.h3, p.ln_w, p.ln_b, y, s.stats, seed, c.stream, c.dry()); }
 }
 
+// The same layer ops as stblock_fwd with no backward state: every intermediate is a workspace transient released once it
+// is dead, so the plan is the live set (h2 under [h1, x0 / stack], then h3 and the LayerNorm statistics where h1 was), and
+// the pre-activations / recurrence planes that only a backward reads are not stored where the kernel can skip them.
+template <class T>
+inline void stblock_infer(const stgcn_stblock_desc& d, const T* x, const stgcn_stblock_params& p, T* y, Ctx c,
+                          uint64_t seed) {
+  StGeom g = st_geom(d);
+  const bool first = d.c_in == 1;
+  const bool q1 = tconv_qonly<T>(g.tc1), q2 = tconv_qonly<T>(g.tc2);
+  ScopedMark sm(c.ws);
+  T* h2 = c.ws.take<T>((size_t)g.rows1 * d.c2);
+  {
+    ScopedMark m1(c.ws);
+    T* h1 = c.ws.take<T>((size_t)g.rows1 * d.c1);
+    {
+      ScopedMark mz(c.ws);
+      T* z1 = tconv_z_optional<T>(g.tc1, q1) ? nullptr : c.ws.take<T>(tconv_saved_elems(g.tc1, q1));
+      Tag t(first ? "st0.tc1.infer" : "st1.tc1.infer");
+      tconv_fwd<T>(g.tc1, x, p.tc1, h1, z1, c, q1);
+    }
+    const bool planes = !gconv_fused<T>(g.gc);
+    T* stack = c.ws.take<T>(planes ? gconv_saved_elems(g.gc) : (size_t)g.rows1 * d.c2);
+    Tag t(first ? "st0.gc.infer" : "st1.gc.infer");
+    gconv_fwd<T>(g.gc, h1, p.gc, h2, stack, c, planes);
+  }
+  T* h3 = c.ws.take<T>((size_t)g.rows2 * d.c3);
+  {
+    ScopedMark mz(c.ws);
+    T* z2 = tconv_z_optional<T>(g.tc2, q2) ? nullptr : c.ws.take<T>(tconv_saved_elems(g.tc2, q2));
+    Tag t(first ? "st0.tc2.infer" : "st1.tc2.infer");
+    tconv_fwd<T>(g.tc2, h2, p.tc2, h3, z2, c, q2);
+  }
+  float* stats = c.ws.take<float>(lnorm_saved_floats(g.ln));
+  Tag t(first ? "st0.ln.infer" : "st1.ln.infer");
+  lnorm_fwd<T>(g.ln, h3, p.ln_w, p.ln_b, y, stats, seed, c.stream, c.dry());
+}
+
 template <class T>
 inline void stblock_bwd(const stgcn_stblock_desc& d, const T* x, Arena& sv, const T* dy,
                         const stgcn_stblock_params& p, const stgcn_stblock_grads& gr, T* dx, Ctx c, uint64_t seed) {
@@ -1064,14 +1130,11 @@ inline bool out_relu_fused(const stgcn_outblock_desc& d, const OutGeom& g) {
   return false;
 }
 
-// y (and dy in the backward) are ALWAYS fp32: the model output feeds the loss (main.py:166-167).
+// fc1 -> ReLU -> dropout -> fc2 of the output block (layers.py:281-284); f1 is unused when the ReLU rides in the fc1
+// epilogue (out_relu_fused)
 template <class T>
-inline void outblock_fwd(const stgcn_outblock_desc& d, const T* x, const stgcn_outblock_params& p, float* y,
-                         Arena& sv, Ctx c, uint64_t seed) {
-  OutGeom g = out_geom(d);
-  OutSaved<T> s = out_saved<T>(d, g, sv);
-  { Tag t("out.tc1.fwd"); tconv_fwd<T>(g.tc, x, p.tc1, s.h, s.z, c, tconv_qonly<T>(g.tc)); }
-  { Tag t("out.ln.fwd"); lnorm_fwd<T>(g.ln, s.h, p.ln_w, p.ln_b, s.l, s.stats, 0, c.stream, c.dry()); }
+inline void out_fc_fwd(const stgcn_outblock_desc& d, const OutGeom& g, const stgcn_outblock_params& p, const T* l, T* f1,
+                       T* r, float* y, Ctx c, uint64_t seed) {
   Tag t_fc("out.fc.fwd");
   ScopedMark sm(c.ws);
   float* w1t = c.K().take<float>((size_t)d.c0 * d.c1);
@@ -1082,13 +1145,13 @@ inline void outblock_fwd(const stgcn_outblock_desc& d, const T* x, const stgcn_o
   auto al16 = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; };
   bool fc1_umma = false;
   if constexpr (std::is_same<T, simt::bf16>::value)
-    fc1_umma = umma_linear(s.l, wbf, p.fc1_b, s.f1, d.B, g.T1, g.T1, d.N, d.c0, d.c1, UmmaLinearOpts{}, c.stream, true);
-  const bool fc2_rowdot = d.c_end == 1 && rowdot_supported(d.c1) && al16(s.r) && g.rows1 > 0;
+    fc1_umma = umma_linear(l, wbf, p.fc1_b, f1, d.B, g.T1, g.T1, d.N, d.c0, d.c1, UmmaLinearOpts{}, c.stream, true);
+  const bool fc2_rowdot = d.c_end == 1 && rowdot_supported(d.c1) && al16(r) && g.rows1 > 0;
   // only the layouts the chosen kernels read are produced
   if (!fc1_umma) launch_gather3(p.fc1_w, w1t, 1, d.c0, d.c1, 0, 0, 1, d.c0, 0, c.ps());      // w1t[c][o] = fc1_w[o][c]
   if (!fc2_rowdot) launch_gather3(p.fc2_w, w2t, 1, d.c1, d.c_end, 0, 0, 1, d.c1, 0, c.ps());
   TapArgs<T> t{};
-  t.in = s.l; t.wt = w1t; t.bias = p.fc1_b; t.out = s.f1; t.rows = g.rows1; t.Cin = d.c0; t.Co = d.c1; t.ntaps = 1;
+  t.in = l; t.wt = w1t; t.bias = p.fc1_b; t.out = f1; t.rows = g.rows1; t.Cin = d.c0; t.Co = d.c1; t.ntaps = 1;
   t.ldo = d.c1; t.map = RowMap{g.T1, g.T1, d.N, 0, 0};
   bool fc1_done = false, relu_done = false;
   if constexpr (std::is_same<T, simt::bf16>::value) {
@@ -1100,24 +1163,61 @@ inline void outblock_fwd(const stgcn_outblock_desc& d, const T* x, const stgcn_o
       UmmaLinearOpts o{};
       relu_done = out_relu_fused<T>(d, g);
       o.relu = relu_done ? 1 : 0;
-      umma_linear(s.l, wbf, p.fc1_b, relu_done ? s.r : s.f1, d.B, g.T1, g.T1, d.N, d.c0, d.c1, o, c.stream, false);
+      umma_linear(l, wbf, p.fc1_b, relu_done ? r : f1, d.B, g.T1, g.T1, d.N, d.c0, d.c1, o, c.stream, false);
       fc1_done = true;
     }
   }
   if (!fc1_done) { c.prep_ready(); launch_tapgemm(t, c.stream); }
   long long n1 = g.rows1 * d.c1;
-  if (n1 && !relu_done) STGCN_LAUNCH(relu_dropout_fwd_kernel<T>, ceil_div(n1, 256), 256, 0, c.stream, (const T*)s.f1, s.r, n1, d.training, d.p_drop, seed);
+  if (n1 && !relu_done) STGCN_LAUNCH(relu_dropout_fwd_kernel<T>, ceil_div(n1, 256), 256, 0, c.stream, (const T*)f1, r, n1, d.training, d.p_drop, seed);
   if (fc2_rowdot) {
     const int lanes = 256 / (d.c1 / 8);
     const int blocks = (int)std::min<long long>(ceil_div(g.rows1, lanes), 148 * 8);
-    STGCN_LAUNCH(rowdot_fwd_kernel<T>, blocks, 256, 0, c.stream, (const T*)s.r, p.fc2_w, p.fc2_b, y, g.rows1, d.c1);
+    STGCN_LAUNCH(rowdot_fwd_kernel<T>, blocks, 256, 0, c.stream, (const T*)r, p.fc2_w, p.fc2_b, y, g.rows1, d.c1);
   } else {
     TapArgs<T, float> t2{};
-    t2.in = s.r; t2.wt = w2t; t2.bias = p.fc2_b; t2.out = y; t2.rows = g.rows1; t2.Cin = d.c1; t2.Co = d.c_end;
+    t2.in = r; t2.wt = w2t; t2.bias = p.fc2_b; t2.out = y; t2.rows = g.rows1; t2.Cin = d.c1; t2.Co = d.c_end;
     t2.ntaps = 1; t2.ldo = d.c_end; t2.map = t.map;
     c.prep_ready();
     launch_tapgemm(t2, c.stream);
   }
+}
+
+// y (and dy in the backward) are ALWAYS fp32: the model output feeds the loss (main.py:166-167).
+template <class T>
+inline void outblock_fwd(const stgcn_outblock_desc& d, const T* x, const stgcn_outblock_params& p, float* y,
+                         Arena& sv, Ctx c, uint64_t seed) {
+  OutGeom g = out_geom(d);
+  OutSaved<T> s = out_saved<T>(d, g, sv);
+  { Tag t("out.tc1.fwd"); tconv_fwd<T>(g.tc, x, p.tc1, s.h, s.z, c, tconv_qonly<T>(g.tc)); }
+  { Tag t("out.ln.fwd"); lnorm_fwd<T>(g.ln, s.h, p.ln_w, p.ln_b, s.l, s.stats, 0, c.stream, c.dry()); }
+  out_fc_fwd<T>(d, g, p, s.l, s.f1, s.r, y, c, seed);
+}
+
+// outblock_fwd with no backward state (see stblock_infer): l under [h, z, statistics], then f1 / r where h was
+template <class T>
+inline void outblock_infer(const stgcn_outblock_desc& d, const T* x, const stgcn_outblock_params& p, float* y, Ctx c,
+                           uint64_t seed) {
+  OutGeom g = out_geom(d);
+  const bool q = tconv_qonly<T>(g.tc);
+  ScopedMark sm(c.ws);
+  T* l = c.ws.take<T>((size_t)g.rows1 * d.c0);
+  {
+    ScopedMark m1(c.ws);
+    T* h = c.ws.take<T>((size_t)g.rows1 * d.c0);
+    {
+      ScopedMark mz(c.ws);
+      T* z = tconv_z_optional<T>(g.tc, q) ? nullptr : c.ws.take<T>(tconv_saved_elems(g.tc, q));
+      Tag t("out.tc1.infer");
+      tconv_fwd<T>(g.tc, x, p.tc1, h, z, c, q);
+    }
+    float* stats = c.ws.take<float>(lnorm_saved_floats(g.ln));
+    Tag t("out.ln.infer");
+    lnorm_fwd<T>(g.ln, h, p.ln_w, p.ln_b, l, stats, 0, c.stream, c.dry());
+  }
+  T* f1 = out_relu_fused<T>(d, g) ? nullptr : c.ws.take<T>((size_t)g.rows1 * d.c1);
+  T* r = c.ws.take<T>((size_t)g.rows1 * d.c1);
+  out_fc_fwd<T>(d, g, p, l, f1, r, y, c, seed);
 }
 
 template <class T>

@@ -299,6 +299,63 @@ int stgcn_outblock_bwd(const stgcn_outblock_desc* d, const void* x, const void* 
   });
 }
 
+// ---------------------------------------------------------------- inference (no backward state)
+int stgcn_stblock_infer_sizes(const stgcn_stblock_desc* d, size_t* workspace_bytes) {
+  return guarded([&] {
+    STGCN_CHECK(d, STGCN_E_INVALID, "null desc");
+    Arena ws(nullptr, 0), keep(nullptr, 0);
+    ops::Ctx c{ws, nullptr};
+    c.keep = &keep;
+    stgcn_stblock_params p{};
+    STGCN_DISPATCH(d->precision, ops::stblock_infer<T>(*d, nullptr, p, nullptr, c, 0));
+    if (workspace_bytes) *workspace_bytes = max2(ws.peak, 256) + Arena::align_up(keep.peak);
+  });
+}
+int stgcn_stblock_infer(const stgcn_stblock_desc* d, const void* x, const stgcn_stblock_params* p, void* y,
+                        void* workspace, size_t workspace_bytes, uint64_t dropout_seed, void* stream) {
+  return guarded([&] {
+    STGCN_CHECK(d && p && x && y && workspace, STGCN_E_INVALID, "null argument");
+    STGCN_DISPATCH(d->precision, run_block(workspace, workspace_bytes, as_stream(stream), [&](ops::Ctx c) {
+                     ops::stblock_infer<T>(*d, (const T*)x, *p, (T*)y, c, dropout_seed);
+                   }));
+  });
+}
+int stgcn_outblock_infer_sizes(const stgcn_outblock_desc* d, size_t* workspace_bytes) {
+  return guarded([&] {
+    STGCN_CHECK(d, STGCN_E_INVALID, "null desc");
+    Arena ws(nullptr, 0), keep(nullptr, 0);
+    ops::Ctx c{ws, nullptr};
+    c.keep = &keep;
+    stgcn_outblock_params p{};
+    STGCN_DISPATCH(d->precision, ops::outblock_infer<T>(*d, nullptr, p, nullptr, c, 0));
+    if (workspace_bytes) *workspace_bytes = max2(ws.peak, 256) + Arena::align_up(keep.peak);
+  });
+}
+int stgcn_outblock_infer(const stgcn_outblock_desc* d, const void* x, const stgcn_outblock_params* p, void* y,
+                         void* workspace, size_t workspace_bytes, uint64_t dropout_seed, void* stream) {
+  return guarded([&] {
+    STGCN_CHECK(d && p && x && y && workspace, STGCN_E_INVALID, "null argument");
+    STGCN_DISPATCH(d->precision, run_block(workspace, workspace_bytes, as_stream(stream), [&](ops::Ctx c) {
+                     ops::outblock_infer<T>(*d, (const T*)x, *p, (float*)y, c, dropout_seed);
+                   }));
+  });
+}
+
+int stgcn_eval_accumulate(const float* pred, const float* target, int32_t B, int32_t N, const float* mean,
+                          const float* scale, double* acc, void* stream) {
+  return guarded([&] {
+    STGCN_CHECK(pred && target && acc, STGCN_E_INVALID, "null argument");
+    STGCN_CHECK(B >= 0 && N > 0, STGCN_E_INVALID, "bad batch geometry");
+    STGCN_CHECK(N <= train::kEvalMaxN, STGCN_E_UNSUPPORTED, "eval_accumulate: N <= 16384");
+    if (B == 0) return;
+    // the opt-in is unconditional: the kernel's static shared memory lowers the default dynamic limit below 48 KB
+    const int smem = (int)(2 * (size_t)N * sizeof(float));
+    STGCN_CUDA(cudaFuncSetAttribute(train::eval_accumulate_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    STGCN_LAUNCH(train::eval_accumulate_kernel, 1, train::kEvalThreads, smem, as_stream(stream), pred, target,
+                 (long long)B * N, (int)N, mean, scale, acc);
+  });
+}
+
 // ---------------------------------------------------------------- diagnostics
 int stgcn_umma_selftest(int mode, const void* A, const void* B, float* C, int M, int N, int K, uint32_t lbo_a,
                         uint32_t sbo_a, uint32_t lbo_b, uint32_t sbo_b, void* stream) {

@@ -84,6 +84,75 @@ __global__ void __launch_bounds__(256) windows_kernel(const float* series, long 
   }
 }
 
+// evaluate_model / evaluate_metric (script/utility.py:90-121) of one batch, summed on the device.  pred, target: [B, N]
+// normalised values.  e = pred - target: acc[0] += e^2.  y / y_pred = StandardScaler.inverse_transform of target / pred on
+// float32 arrays (x * scale[n], then + mean[n], each rounded to float32, no FMA contraction); d = |y - y_pred|:
+// acc[1] += d, acc[2] += d^2 (float32, as numpy squares it), acc[3] += y.  ONE CTA: every thread sums its elements in fp64
+// in an order fixed by (B, N), then a fixed-order block reduction and a single plain read-modify-write of acc -- no
+// atomics, bit-reproducible, capturable.  The per-node mean / scale are staged in shared memory once.
+constexpr int kEvalThreads = 1024;
+constexpr int kEvalMaxN = 16384;          // 2 x N floats of shared memory
+
+__device__ __forceinline__ void eval_one(float p, float t, int n, const float* mean_s, const float* scale_s, bool hm, bool hs,
+                                         double (&a)[4]) {
+  const float e = __fsub_rn(p, t);
+  a[0] += (double)__fmul_rn(e, e);
+  float y = t, yp = p;
+  if (hs) { y = __fmul_rn(y, scale_s[n]); yp = __fmul_rn(yp, scale_s[n]); }
+  if (hm) { y = __fadd_rn(y, mean_s[n]); yp = __fadd_rn(yp, mean_s[n]); }
+  const float d = fabsf(__fsub_rn(y, yp));
+  a[1] += (double)d;
+  a[2] += (double)__fmul_rn(d, d);
+  a[3] += (double)y;
+}
+
+__global__ void __launch_bounds__(kEvalThreads) eval_accumulate_kernel(const float* pred, const float* target, long long n,
+                                                                       int N, const float* mean, const float* scale,
+                                                                       double* acc) {
+  extern __shared__ float eval_s[];                 // [N] mean, [N] scale
+  __shared__ double red[kEvalThreads / 32][4];
+  const bool hm = mean != nullptr, hs = scale != nullptr;
+  float* mean_s = eval_s;
+  float* scale_s = eval_s + N;
+  for (int i = threadIdx.x; i < N; i += blockDim.x) {
+    if (hm) mean_s[i] = mean[i];
+    if (hs) scale_s[i] = scale[i];
+  }
+  __syncthreads();
+  double a[4] = {0.0, 0.0, 0.0, 0.0};
+  const bool vec = ((reinterpret_cast<uintptr_t>(pred) | reinterpret_cast<uintptr_t>(target)) & 15) == 0;
+  const long long n8 = vec ? n / 8 : 0;
+  for (long long c = threadIdx.x; c < n8; c += blockDim.x) {        // 8 elements per step, 16-byte loads
+    const float4* p4 = reinterpret_cast<const float4*>(pred) + 2 * c;
+    const float4* t4 = reinterpret_cast<const float4*>(target) + 2 * c;
+    const float4 p0 = p4[0], p1 = p4[1], t0 = t4[0], t1 = t4[1];
+    const float pv[8] = {p0.x, p0.y, p0.z, p0.w, p1.x, p1.y, p1.z, p1.w};
+    const float tv[8] = {t0.x, t0.y, t0.z, t0.w, t1.x, t1.y, t1.z, t1.w};
+    int node = (int)((c * 8) % N);
+#pragma unroll
+    for (int k = 0; k < 8; ++k) {
+      eval_one(pv[k], tv[k], node, mean_s, scale_s, hm, hs, a);
+      if (++node == N) node = 0;
+    }
+  }
+  for (long long i = n8 * 8 + threadIdx.x; i < n; i += blockDim.x)   // tail (B*N % 8) or unaligned buffers
+    eval_one(pred[i], target[i], (int)(i % N), mean_s, scale_s, hm, hs, a);
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int k = 0; k < 4; ++k)
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) a[k] += __shfl_down_sync(0xffffffffu, a[k], o);
+  if (lane == 0)
+#pragma unroll
+    for (int k = 0; k < 4; ++k) red[warp][k] = a[k];
+  __syncthreads();
+  if (threadIdx.x < 4) {
+    double s = 0.0;
+    for (int w = 0; w < (int)(blockDim.x >> 5); ++w) s += red[w][threadIdx.x];
+    acc[threadIdx.x] += s;
+  }
+}
+
 inline int elementwise_grid(long long work_items) {
   long long blocks = (work_items + 255) / 256;
   const long long cap = 148LL * 8;

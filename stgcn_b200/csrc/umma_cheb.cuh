@@ -62,7 +62,8 @@ struct ChebParams {
   const bf16* a_mat;                    // operator, bf16 [N][Kp] zero padded (gso_prep_kernel; transposed for backward)
   const float* w;                       // [n_taps][16][16] fp32 (c_in, c_out)
   const float* bias;                    // [16] or nullptr
-  // forward: in = x_0 plane (= stack plane 0), stack = [depth][G][N][16] (planes 1.. written), out = y
+  // forward: in = x_0 plane (= stack plane 0), stack = [depth][G][N][16] (planes 1.. written) or nullptr (inference:
+  // planes 1.. only in shared memory, as the next hop's operand), out = y
   // backward: in = dy, in2 = y, out = dx_0, out2 = dG
   const bf16* in; const bf16* in2; bf16* stack; bf16* out; bf16* out2;
   unsigned long long* dbg;              // optional timeline stamps (diagnostics)
@@ -312,7 +313,7 @@ __global__ void __launch_bounds__(kChebThreads, 1) umma_cheb_kernel(ChebParams p
             const float alpha = k == 1 ? 1.f : 2.f;
             uint8_t* bk = bufs + (size_t)(k + 1) * p.buf_bytes;
             const uint8_t* bm2 = k == 2 ? x0b : bufs + (size_t)(k >= 2 ? k - 1 : 0) * p.buf_bytes;
-            bf16* plane = p.stack + (size_t)k * p.plane;
+            bf16* plane = p.stack ? p.stack + (size_t)k * p.plane : nullptr;     // null: inference, x_k stays in smem
             mbar_wait(acc_full, n_acc & 1); ++n_acc;
             tc_fence_after();
             if (stamp) CHEB_STAMP(8 + 2 * (k - 1));
@@ -344,7 +345,7 @@ __global__ void __launch_bounds__(kChebThreads, 1) umma_cheb_kernel(ChebParams p
                   }
                   const uint4 lo = pack8_bf16(v), hi = pack8_bf16(v + 8);
                   if (inbuf) row_store(bk + (size_t)g * p.gs, n, lo, hi);
-                  if (nvalid && g0 + g < p.G) {
+                  if (plane && nvalid && g0 + g < p.G) {
                     uint4* dst = reinterpret_cast<uint4*>(plane + ((g0 + g) * p.N + n) * kChebC);
                     dst[0] = lo; dst[1] = hi;
                   }

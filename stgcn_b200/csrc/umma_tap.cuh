@@ -257,7 +257,9 @@ __device__ __forceinline__ void tap_issue(uint32_t d_tmem, uint64_t da, uint64_t
     }
   }
 }
-template <int EPI, int ACT, bool AUX>
+// KZ: the gate epilogue keeps the pre-activation (out_z, the training forward); false = inference, no Q / z stores.  A
+// template parameter, so the training instantiations compile to exactly the code they had without the inference variant.
+template <int EPI, int ACT, bool AUX, bool KZ = true>
 __global__ void __launch_bounds__(kTapThreadsWide, 1)
 umma_tap_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmW,
                 const __grid_constant__ CUtensorMap tmO, const __grid_constant__ CUtensorMap tmZ, TapParams p) {
@@ -636,8 +638,10 @@ umma_tap_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
                 wq[k] = pack_bf16x2(q0, q1);
                 wh[k] = pack_bf16x2(h0, h1);
               }
-              asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(o0), "r"(wq[0]), "r"(wq[1]), "r"(wq[2]), "r"(wq[3]) : "memory");
-              asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(o1), "r"(wq[4]), "r"(wq[5]), "r"(wq[6]), "r"(wq[7]) : "memory");
+              if (KZ) {                                    // inference (KZ = false): nZ = 0, no Q sub-tiles
+                asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(o0), "r"(wq[0]), "r"(wq[1]), "r"(wq[2]), "r"(wq[3]) : "memory");
+                asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(o1), "r"(wq[4]), "r"(wq[5]), "r"(wq[6]), "r"(wq[7]) : "memory");
+              }
               asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(o0 + h_off), "r"(wh[0]), "r"(wh[1]), "r"(wh[2]), "r"(wh[3]) : "memory");
               asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(o1 + h_off), "r"(wh[4]), "r"(wh[5]), "r"(wh[6]), "r"(wh[7]) : "memory");
             }
@@ -740,7 +744,8 @@ umma_tap_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
               for (int i = 0; i < 8; ++i) h[i] = epi_act<ACT>((AUX && has_aux) ? zp[i] + av[i] : zp[i], zq[i]);
               const uint4 oh = pack8_bf16(h);
               if (stg) {
-                if (gated && p.q_only) {
+                if (!KZ) {
+                } else if (gated && p.q_only) {
                   stage_store8_s(sub, row, c8 & 63, pack8_bf16(zq));
                 } else {
                   stage_store8_s(sub, row, c8 & 63, pack8_bf16(zp));
@@ -749,7 +754,8 @@ umma_tap_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__
                 stage_store8_s(stg_s + (uint32_t)(p.nZ + (c8 >> 6)) * 16384u, row, c8 & 63, oh);
               } else if (valid) {
                 const long long orow = ((long long)b * p.T_out + t_o) * p.N + n;
-                if (gated && p.q_only) {
+                if (!KZ) {
+                } else if (gated && p.q_only) {
                   *reinterpret_cast<uint4*>(p.out_z + orow * p.Cout + c8) = pack8_bf16(zq);
                 } else {
                   *reinterpret_cast<uint4*>(p.out_z + orow * p.W + c8) = pack8_bf16(zp);
@@ -813,7 +819,7 @@ struct TapProblem {
   int epi, act, Cout;      // gate: Co == W
   const bf16* aux; int aux_dt, T_aux, C_aux, aux_cols;
   bf16* out; int ld_out;
-  bf16* out_z;
+  bf16* out_z;             // gate: saved pre-activation, or nullptr (inference: nothing a backward would read is stored)
   int q_only;              // gate (GLU): store only the Q half of z ([rows, Cout])
   // optional element strides of `in` for the vertex / time / batch axes (0 = dense [B,T_src,N,Cin]); lets a stack of
   // planes [Kt][B*T][N][C] be read with the plane index as the "time" axis
@@ -917,6 +923,17 @@ inline int sm_count() {
   return n;
 }
 
+// Gate epilogues that have no inference (KZ = false) instantiation: GLU / GTU with the residual in the epilogue (AUX) --
+// without the z stores ptxas spills more there (96 / 160 / 216 B frame / stores / loads instead of 80 / 120 / 140), so
+// the inference chain keeps z in its workspace for them (ops.cuh: tconv_z_optional).
+inline bool tap_nz_spills(int act, bool aux_epi) { return aux_epi && (act == STGCN_ACT_GLU || act == STGCN_ACT_GTU); }
+// whether launch_tap runs the residual in the epilogue (shapes only; `in` and `aux` are the same tensor, as in tconv_fwd)
+inline bool tap_aux_epilogue(const TapProblem& q) {
+  if (q.aux == nullptr) return false;
+  TapPlan pl = plan_tap(q.Cin, q.Co, q.Kt, q.T_src, q.epi == EPI_GATE, q.Cout, q.q_only != 0, tap_want_bias(q), tap_want_res(q));
+  return !pl.res_mma;
+}
+
 inline void launch_tap(const TapProblem& q, cudaStream_t stream) {
   TapPlan pl = plan_tap(q.Cin, q.Co, q.Kt, q.T_src, q.epi == EPI_GATE, q.Cout, q.q_only != 0, tap_want_bias(q), tap_want_res(q));
   STGCN_CHECK(pl.ok, STGCN_E_UNSUPPORTED, "umma tap GEMM: unsupported shape");
@@ -942,7 +959,7 @@ inline void launch_tap(const TapProblem& q, cudaStream_t stream) {
     uint64_t os[3] = {(uint64_t)Cmain * 2, (uint64_t)q.N * Cmain * 2, (uint64_t)q.T_out * q.N * Cmain * 2};
     uint32_t ob[4] = {64, 128, 1, 1};
     tmO = make_tmap_bf16(q.out, 4, od, os, ob, CU_TENSOR_MAP_SWIZZLE_128B);
-    if (q.epi == EPI_GATE) {
+    if (q.epi == EPI_GATE && q.out_z) {
       const uint64_t zc = q.q_only ? q.Cout : q.Co;        // channels per row of the saved tensor
       uint64_t zd[4] = {zc, (uint64_t)q.N, (uint64_t)q.T_out, (uint64_t)q.B};
       uint64_t zs[3] = {zc * 2, (uint64_t)q.N * zc * 2, (uint64_t)q.T_out * q.N * zc * 2};
@@ -950,7 +967,10 @@ inline void launch_tap(const TapProblem& q, cudaStream_t stream) {
     }
   }
   TapParams p{};
-  p.store_tma = pl.store_tma; p.nbuf = pl.nbuf; p.nZ = pl.nZ; p.nO = pl.nO; p.stage_off = pl.stage_off;
+  // gate without out_z (inference, umma_tap_kernel<..., KZ = false>): the plan -- and with it the per-element arithmetic --
+  // stays the forward's; only the Q sub-tiles are neither staged nor stored, and the H sub-tiles move to stage offset 0
+  p.store_tma = pl.store_tma; p.nbuf = pl.nbuf; p.nZ = (q.epi == EPI_GATE && !q.out_z) ? 0 : pl.nZ; p.nO = pl.nO;
+  p.stage_off = pl.stage_off;
   p.stage_bytes = pl.stage_bytes;
   p.B = q.B; p.N = q.N; p.T_src = q.T_src; p.T_out = q.T_out; p.Kt = q.Kt; p.t0 = q.t0;
   p.Cin = q.Cin; p.KB = pl.KB; p.nKB = pl.nKB; p.CoT = pl.CoT; p.S = pl.S; p.swz = pl.swz; p.sbo = pl.sbo;
@@ -1019,19 +1039,29 @@ inline void launch_tap(const TapProblem& q, cudaStream_t stream) {
     STGCN_LAUNCH_NAMED(kname, kern, grid, kTapThreadsWide, pl.smem, stream, tmX, tmW, tmO, tmZ, p);
   };
   const bool aux_epi = p.aux != nullptr;
-#define STGCN_TAP_GO(EPIV, ACTV) do { if (aux_epi) go(umma_tap_kernel<EPIV, ACTV, true>); else go(umma_tap_kernel<EPIV, ACTV, false>); } while (0)
+  const bool keep_z = q.epi != EPI_GATE || q.out_z != nullptr;
+  STGCN_CHECK(keep_z || !tap_nz_spills(q.act, aux_epi), STGCN_E_INVALID, "umma tap GEMM: this gate needs out_z");
+#define STGCN_TAP_GO(EPIV, ACTV) do {                                                                   \
+    if (keep_z) { if (aux_epi) go(umma_tap_kernel<EPIV, ACTV, true>); else go(umma_tap_kernel<EPIV, ACTV, false>); } \
+    else { if (aux_epi) go(umma_tap_kernel<EPIV, ACTV, true, false>); else go(umma_tap_kernel<EPIV, ACTV, false, false>); } \
+  } while (0)
+#define STGCN_TAP_GO_KZ(EPIV, ACTV) do {                                                                \
+    if (aux_epi) go(umma_tap_kernel<EPIV, ACTV, true>); else if (keep_z) go(umma_tap_kernel<EPIV, ACTV, false>);   \
+    else go(umma_tap_kernel<EPIV, ACTV, false, false>);                                                \
+  } while (0)
   if (q.epi == EPI_GATE) {
     switch (q.act) {
-      case STGCN_ACT_GLU: STGCN_TAP_GO(EPI_GATE, STGCN_ACT_GLU); break;
-      case STGCN_ACT_GTU: STGCN_TAP_GO(EPI_GATE, STGCN_ACT_GTU); break;
+      case STGCN_ACT_GLU: STGCN_TAP_GO_KZ(EPI_GATE, STGCN_ACT_GLU); break;
+      case STGCN_ACT_GTU: STGCN_TAP_GO_KZ(EPI_GATE, STGCN_ACT_GTU); break;
       case STGCN_ACT_RELU: STGCN_TAP_GO(EPI_GATE, STGCN_ACT_RELU); break;
       case STGCN_ACT_SILU: STGCN_TAP_GO(EPI_GATE, STGCN_ACT_SILU); break;
       default: STGCN_TAP_GO(EPI_GATE, STGCN_ACT_LINEAR); break;
     }
   } else {
-    STGCN_TAP_GO(EPI_LINEAR, STGCN_ACT_LINEAR);
+    if (aux_epi) go(umma_tap_kernel<EPI_LINEAR, STGCN_ACT_LINEAR, true>); else go(umma_tap_kernel<EPI_LINEAR, STGCN_ACT_LINEAR, false>);
   }
 #undef STGCN_TAP_GO
+#undef STGCN_TAP_GO_KZ
 }
 
 }  // namespace umma

@@ -368,6 +368,56 @@ class _OutBlockFn(torch.autograd.Function):
 
 
 # ----------------------------------------------------------------------------------------------
+# inference (no autograd node, no backward state: stgcn_*_infer)
+# ----------------------------------------------------------------------------------------------
+def _no_backward(x: torch.Tensor, params) -> bool:
+    """True when autograd will never ask for this block's backward: grad mode is off (torch.no_grad(), inference_mode(),
+    evaluate_model / evaluate_metric) or neither the input nor any parameter requires grad."""
+    if not torch.is_grad_enabled():
+        return True
+    return not (x.requires_grad or any(p is not None and p.requires_grad for p in params))
+
+
+def _stblock_infer(x_cl, dims, gso, params):
+    """STConvBlock forward through stgcn_stblock_infer: the result of _STBlockFn.forward, bit for bit, without the
+    saved buffer; same workspace cache and dropout-seed rule."""
+    (B, T, N, c_in, c1, c2, c3, Kt, Ks, act, gconv, training, p_drop, eps) = dims
+    lib = L.lib()
+    desc = L.StblockDesc(B, T, N, c_in, c1, c2, c3, Kt, Ks, act, gconv, int(training), float(p_drop), float(eps),
+                         L.PREC[_PRECISION])
+    ws_bytes = C.c_size_t(0)
+    L.check(lib.stgcn_stblock_infer_sizes(C.byref(desc), C.byref(ws_bytes)))
+    dev = x_cl.device
+    ws = _workspace(dev, int(ws_bytes.value))
+    y = torch.empty((B, T - 2 * (Kt - 1), N, c3), dtype=x_cl.dtype, device=dev)
+    seed = _next_seed() if (training and p_drop > 0) else 0
+    cparams = _STBlockFn._pack(params, gso)
+    with torch.cuda.device(dev):      # kernels, helper streams and events follow the CUDA current device
+        L.check(lib.stgcn_stblock_infer(C.byref(desc), x_cl.data_ptr(), C.byref(cparams), y.data_ptr(), ws.data_ptr(),
+                                        ws.numel(), seed, _stream(dev)))
+    return y
+
+
+def _outblock_infer(x_cl, dims, params):
+    """OutputBlock forward through stgcn_outblock_infer (see _stblock_infer)."""
+    (B, T, N, c_in, c0, c1, c_end, Ko, act, training, p_drop, eps) = dims
+    lib = L.lib()
+    desc = L.OutblockDesc(B, T, N, c_in, c0, c1, c_end, Ko, act, int(training), float(p_drop), float(eps),
+                          L.PREC[_PRECISION])
+    ws_bytes = C.c_size_t(0)
+    L.check(lib.stgcn_outblock_infer_sizes(C.byref(desc), C.byref(ws_bytes)))
+    dev = x_cl.device
+    ws = _workspace(dev, int(ws_bytes.value))
+    y = torch.empty((B, T - Ko + 1, N, c_end), dtype=torch.float32, device=dev)
+    seed = _next_seed() if (training and p_drop > 0) else 0
+    cparams = _OutBlockFn._pack(params)
+    with torch.cuda.device(dev):      # kernels, helper streams and events follow the CUDA current device
+        L.check(lib.stgcn_outblock_infer(C.byref(desc), x_cl.data_ptr(), C.byref(cparams), y.data_ptr(), ws.data_ptr(),
+                                         ws.numel(), seed, _stream(dev)))
+    return y
+
+
+# ----------------------------------------------------------------------------------------------
 # modules (names, ctor signatures and parameter names of the reference)
 # ----------------------------------------------------------------------------------------------
 def _act_code(act_func: str) -> int:
@@ -614,6 +664,8 @@ class STConvBlock(nn.Module):
                 L.GCONV[gc.graph_conv_type], self.training, self.dropout.p, self.tc2_ln.eps)
         params = (*_tconv_param_tuple(t1), *gc._params(), *_tconv_param_tuple(t2),
                   _f32c(self.tc2_ln.weight), _f32c(self.tc2_ln.bias))
+        if _no_backward(x, params):
+            return _as_bctn(_stblock_infer(_channels_last(x), dims, gc.gso, params))
         return _as_bctn(_STBlockFn.apply(_channels_last(x), dims, gc.gso, *params))
 
 
@@ -640,4 +692,6 @@ class OutputBlock(nn.Module):
                 self.dropout.p, self.tc1_ln.eps)
         params = (*_tconv_param_tuple(t1), _f32c(self.tc1_ln.weight), _f32c(self.tc1_ln.bias),
                   _f32c(self.fc1.weight), _f32c(self.fc1.bias), _f32c(self.fc2.weight), _f32c(self.fc2.bias))
+        if _no_backward(x, params):
+            return _as_bctn(_outblock_infer(_channels_last(x), dims, params))
         return _as_bctn(_OutBlockFn.apply(_channels_last(x), dims, *params))
