@@ -266,6 +266,16 @@ int stgcn_mse_fwd_bwd(const float* pred, const float* target, int64_t n, float l
 int stgcn_adamw_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, int64_t n,
                      float lr, float beta1, float beta2, float eps, float weight_decay, float grad_scale,
                      int64_t step, const int64_t* step_dev, const float* lr_dev, void* stream);
+/* Same for torch.optim.NAdam(decoupled_weight_decay=True), the reference's `--opt nadamw` (main.py:149-150): replaces
+ * its per-tensor optimizer.step() with one launch.  Arguments as stgcn_adamw_step, plus momentum_decay (psi) and
+ * mu_product: device float[2], the float32 product of the momentum caches mu_1 .. mu_t that torch keeps per parameter
+ * (one scalar here: every live parameter has the same step count).  Step t reads slot (t-1)&1 and writes slot t&1, so
+ * that no thread of a launch reads the value it publishes; initialise slot 0 to 1 before step 1.  The step scalars are
+ * computed in fp64, as torch computes them in Python floats.                                                      */
+int stgcn_nadamw_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, int64_t n,
+                      float lr, float beta1, float beta2, float eps, float weight_decay, float grad_scale,
+                      int64_t step, const int64_t* step_dev, const float* lr_dev, float momentum_decay,
+                      float* mu_product, void* stream);
 /* same for the reference's Lion optimizer (script/opt.py:34-76)                                                 */
 int stgcn_lion_step(float* params, const float* grads, float* exp_avg, int64_t n, float lr, float beta1,
                     float beta2, float weight_decay, float grad_scale, const float* lr_dev, void* stream);

@@ -130,6 +130,8 @@ _SIGNATURES = [
     ("stgcn_mse_fwd_bwd", C.c_int, [_fp, _fp, C.c_int64, C.c_float, _fp, _fp, _fp]),
     ("stgcn_adamw_step", C.c_int, [_fp, _fp, _fp, _fp, C.c_int64, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float,
                                    C.c_float, C.c_int64, _fp, _fp, _fp]),
+    ("stgcn_nadamw_step", C.c_int, [_fp, _fp, _fp, _fp, C.c_int64, C.c_float, C.c_float, C.c_float, C.c_float,
+                                    C.c_float, C.c_float, C.c_int64, _fp, _fp, C.c_float, _fp, _fp]),
     ("stgcn_lion_step", C.c_int, [_fp, _fp, _fp, C.c_int64, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, _fp,
                                   _fp]),
     ("stgcn_gso_build", C.c_int, [_fp, C.c_int32, C.c_int32, C.c_int32, _fp, _fp, _fp, _sz, _fp]),

@@ -411,6 +411,23 @@ int stgcn_adamw_step(float* params, const float* grads, float* exp_avg, float* e
     STGCN_LAUNCH(train::adamw_kernel, train::elementwise_grid((n + 3) / 4), 256, 0, as_stream(stream), a);
   });
 }
+int stgcn_nadamw_step(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, int64_t n, float lr,
+                      float beta1, float beta2, float eps, float weight_decay, float grad_scale, int64_t step,
+                      const int64_t* step_dev, const float* lr_dev, float momentum_decay, float* mu_product,
+                      void* stream) {
+  return guarded([&] {
+    STGCN_CHECK(params && grads && exp_avg && exp_avg_sq && mu_product && n >= 0, STGCN_E_INVALID, "null argument");
+    STGCN_CHECK(step >= 1 || step_dev, STGCN_E_INVALID, "NAdamW step numbers start at 1");
+    if (n == 0) return;
+    auto al16 = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; };
+    STGCN_CHECK(al16(params) && al16(grads) && al16(exp_avg) && al16(exp_avg_sq), STGCN_E_INVALID,
+                "flat optimizer buffers must be 16-byte aligned");
+    train::NAdamWArgs a{params, grads, exp_avg, exp_avg_sq, (long long)n, lr, beta1, beta2, eps, weight_decay,
+                        grad_scale, momentum_decay, (long long)step, reinterpret_cast<const long long*>(step_dev), lr_dev,
+                        mu_product};
+    STGCN_LAUNCH(train::nadamw_kernel, train::elementwise_grid((n + 3) / 4), 256, 0, as_stream(stream), a);
+  });
+}
 int stgcn_lion_step(float* params, const float* grads, float* exp_avg, int64_t n, float lr, float beta1, float beta2,
                     float weight_decay, float grad_scale, const float* lr_dev, void* stream) {
   return guarded([&] {

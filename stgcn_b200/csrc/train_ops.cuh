@@ -51,6 +51,66 @@ __global__ void __launch_bounds__(256) adamw_kernel(AdamWArgs a) {
   }
 }
 
+struct NAdamWArgs {
+  float* p; const float* g; float* m; float* v;
+  long long n;
+  float lr, beta1, beta2, eps, wd, grad_scale, momentum_decay;
+  long long step;                       // 1-based step number, or *step_dev + 1 when step_dev is non-null
+  const long long* step_dev;
+  const float* lr_dev;
+  float* mu_product;                    // [2] ping-pong slots of the float32 momentum-cache product (see below)
+};
+
+// torch.optim.NAdam(decoupled_weight_decay=True), the reference's `--opt nadamw` (main.py:149-150), as
+// _single_tensor_nadam computes it at step t: p *= 1 - lr*wd; m = lerp(m, g, 1-b1); v = b2 v + (1-b2) g^2;
+// mu_t = b1 (1 - 0.5 * 0.96^(t psi)); Pi_t = Pi_{t-1} * mu_t (float32, as torch's mu_product state);
+// denom = sqrt(v / (1 - b2^t)) + eps; p += c_g * g / denom + c_m * m / denom with
+// c_g = -lr (1 - mu_t) / (1 - Pi_t), c_m = -lr mu_{t+1} / (1 - Pi_t mu_{t+1}).  The step scalars are fp64, as torch's
+// Python floats; every element-wise product is fp32, as torch's tensor ops.
+__device__ __forceinline__ void nadamw_one(float& p, float g, float& m, float& v, float decay, float one_m_b1, float b2,
+                                           float one_m_b2, float bc2, float eps, float c_g, float c_m) {
+  p *= decay;
+  m = fmaf(one_m_b1, g - m, m);            // torch: exp_avg.lerp_(grad, 1 - beta1)
+  v = b2 * v + one_m_b2 * g * g;           // torch: exp_avg_sq.mul_(beta2).addcmul_(grad, grad, value=1 - beta2)
+  const float denom = sqrtf(v / bc2) + eps;
+  p += c_g * g / denom;                    // torch: param.addcdiv_(grad, denom, value=c_g)
+  p += c_m * m / denom;                    //        param.addcdiv_(exp_avg, denom, value=c_m)
+}
+// Pi is one scalar shared by every parameter (all live parameters have the same step count).  Every thread needs
+// Pi_{t-1} and exactly one write may publish Pi_t, so the product ping-pongs between two slots by step parity: step t
+// reads slot (t-1)&1 and thread 0 of block 0 writes slot t&1, which no thread of the same launch reads.  The next
+// launch reads it after stream ordering has made the write visible.  The caller initialises slot 0 to Pi_0 = 1.
+__global__ void __launch_bounds__(256) nadamw_kernel(NAdamWArgs a) {
+  const long long t = a.step_dev ? *a.step_dev + 1 : a.step;
+  const double lr = a.lr_dev ? (double)*a.lr_dev : (double)a.lr;
+  const double b1 = a.beta1, psi = a.momentum_decay;
+  const double mu = b1 * (1.0 - 0.5 * pow(0.96, (double)t * psi));
+  const double mu_next = b1 * (1.0 - 0.5 * pow(0.96, (double)(t + 1) * psi));
+  const float prod = a.mu_product[(t - 1) & 1] * (float)mu;          // torch: mu_product (float32) *= mu
+  if (blockIdx.x == 0 && threadIdx.x == 0) a.mu_product[t & 1] = prod;
+  const float c_g = (float)(-lr * (1.0 - mu) / (1.0 - (double)prod));
+  const float c_m = (float)(-lr * mu_next / (1.0 - (double)prod * mu_next));
+  const float bc2 = (float)(1.0 - pow((double)a.beta2, (double)t));
+  const float decay = (float)(1.0 - lr * (double)a.wd);
+  const float one_m_b1 = (float)(1.0 - b1), one_m_b2 = (float)(1.0 - (double)a.beta2);
+  const long long n4 = a.n >> 2, stride = (long long)gridDim.x * blockDim.x;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
+    float4 p = reinterpret_cast<float4*>(a.p)[i], m = reinterpret_cast<float4*>(a.m)[i], v = reinterpret_cast<float4*>(a.v)[i];
+    float4 g = reinterpret_cast<const float4*>(a.g)[i];
+    g.x *= a.grad_scale; g.y *= a.grad_scale; g.z *= a.grad_scale; g.w *= a.grad_scale;
+    nadamw_one(p.x, g.x, m.x, v.x, decay, one_m_b1, a.beta2, one_m_b2, bc2, a.eps, c_g, c_m);
+    nadamw_one(p.y, g.y, m.y, v.y, decay, one_m_b1, a.beta2, one_m_b2, bc2, a.eps, c_g, c_m);
+    nadamw_one(p.z, g.z, m.z, v.z, decay, one_m_b1, a.beta2, one_m_b2, bc2, a.eps, c_g, c_m);
+    nadamw_one(p.w, g.w, m.w, v.w, decay, one_m_b1, a.beta2, one_m_b2, bc2, a.eps, c_g, c_m);
+    reinterpret_cast<float4*>(a.p)[i] = p; reinterpret_cast<float4*>(a.m)[i] = m; reinterpret_cast<float4*>(a.v)[i] = v;
+  }
+  for (long long i = (n4 << 2) + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < a.n; i += stride) {
+    float p = a.p[i], m = a.m[i], v = a.v[i];
+    nadamw_one(p, a.g[i] * a.grad_scale, m, v, decay, one_m_b1, a.beta2, one_m_b2, bc2, a.eps, c_g, c_m);
+    a.p[i] = p; a.m[i] = m; a.v[i] = v;
+  }
+}
+
 // Lion (script/opt.py:34-76): p *= 1 - lr*wd; p -= lr * sign(b1 m + (1-b1) g); m = b2 m + (1-b2) g
 __global__ void __launch_bounds__(256) lion_kernel(float* p, const float* g, float* m, long long n, float lr,
                                                    const float* lr_dev, float b1, float b2, float wd, float grad_scale) {
