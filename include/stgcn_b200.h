@@ -88,6 +88,21 @@ typedef struct {
 
 typedef struct { float* align_w; float* align_b; float* w; float* b; } stgcn_gconv_grads;
 
+/* A sparse graph shift operator in CSR form (device arrays), the operator the reference builds as a scipy sparse
+ * matrix (script/utility.py:6-76) before densifying it (main.py:101).  Row h holds entries row_ptr[h] ..
+ * row_ptr[h+1]-1 with column col[j] and value val[j]; the t_* arrays hold gso^T the same way (the backward's adjoint
+ * recurrence reads them) and may alias the forward arrays when the operator is symmetric.  Columns must lie in [0, N).
+ * Duplicate entries are summed in storage order.  stgcn_b200.gso.CsrOperator builds this from scipy / torch.        */
+typedef struct {
+  int32_t N, nnz;
+  const int32_t* row_ptr;   /* [N + 1], row_ptr[0] = 0, row_ptr[N] = nnz */
+  const int32_t* col;       /* [nnz] */
+  const float* val;         /* [nnz] */
+  const int32_t* t_row_ptr; /* gso^T: [N + 1] */
+  const int32_t* t_col;     /* [nnz] */
+  const float* t_val;       /* [nnz] */
+} stgcn_csr_gso;
+
 /* ---- LayerNorm over (N, C) per (b, t) + dropout (layers.py:246-248,255-256) ---------- */
 typedef struct {
   int32_t B, T, N, C;
@@ -224,6 +239,34 @@ int stgcn_stblock_infer(const stgcn_stblock_desc*, const void* x, const stgcn_st
 int stgcn_outblock_infer_sizes(const stgcn_outblock_desc*, size_t* workspace_bytes);
 int stgcn_outblock_infer(const stgcn_outblock_desc*, const void* x, const stgcn_outblock_params*, void* y,
                          void* workspace, size_t workspace_bytes, uint64_t dropout_seed, void* stream);
+/* ---- sparse graph shift operators: the entry points above that read a gso, with a CSR operator ------------------ */
+/* Each *_csr twin takes the arguments of its dense counterpart plus `op`, and replaces the same reference code; the
+ * node contraction -- the einsums over gso of ChebGraphConv / GraphConv.forward (layers.py:154-165, 198-199) -- runs
+ * as a CSR SpMM over the (B*T, N, C) planes instead of a dense (N, N) product, and the dense bf16 operator image is not
+ * reserved in the workspace.  params->gc.gso (params->gso for the layer calls) must be NULL; op->N must equal the
+ * desc's N; op->nnz >= 0; the two row-offset arrays must be non-NULL, and the four column / value arrays too when
+ * nnz > 0 (the size queries only check them).  Otherwise STGCN_E_INVALID.  The saved
+ * buffer of *_fwd_csr must be passed to *_bwd_csr with the same op.  Deterministic (no atomics).                   */
+int stgcn_gconv_sizes_csr(const stgcn_gconv_desc*, const stgcn_csr_gso* op, size_t* saved_bytes,
+                          size_t* workspace_bytes);
+int stgcn_gconv_fwd_csr(const stgcn_gconv_desc*, const void* x, const stgcn_gconv_params*, const stgcn_csr_gso* op,
+                        void* y, void* saved, void* workspace, size_t workspace_bytes, void* stream);
+int stgcn_gconv_bwd_csr(const stgcn_gconv_desc*, const void* x, const void* saved, const void* dy,
+                        const stgcn_gconv_params*, const stgcn_csr_gso* op, const stgcn_gconv_grads*, void* dx,
+                        void* workspace, size_t workspace_bytes, void* stream);
+int stgcn_stblock_sizes_csr(const stgcn_stblock_desc*, const stgcn_csr_gso* op, size_t* saved_bytes,
+                            size_t* workspace_bytes);
+int stgcn_stblock_fwd_csr(const stgcn_stblock_desc*, const void* x, const stgcn_stblock_params*,
+                          const stgcn_csr_gso* op, void* y, void* saved, void* workspace, size_t workspace_bytes,
+                          uint64_t dropout_seed, void* stream);
+int stgcn_stblock_bwd_csr(const stgcn_stblock_desc*, const void* x, const void* saved, const void* dy,
+                          const stgcn_stblock_params*, const stgcn_csr_gso* op, const stgcn_stblock_grads*, void* dx,
+                          void* workspace, size_t workspace_bytes, uint64_t dropout_seed, void* stream);
+int stgcn_stblock_infer_sizes_csr(const stgcn_stblock_desc*, const stgcn_csr_gso* op, size_t* workspace_bytes);
+int stgcn_stblock_infer_csr(const stgcn_stblock_desc*, const void* x, const stgcn_stblock_params*,
+                            const stgcn_csr_gso* op, void* y, void* workspace, size_t workspace_bytes,
+                            uint64_t dropout_seed, void* stream);
+
 /* evaluate_model / evaluate_metric (script/utility.py:90-121) of one batch, accumulated on the device.  pred, target:
  * (B, N) fp32, normalised.  acc: device double[4], zeroed by the caller, to which this adds
  *   acc[0] += sum (pred - target)^2                      (the MSELoss of evaluate_model, on normalised values)

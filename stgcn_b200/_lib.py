@@ -91,6 +91,12 @@ class OutblockGrads(C.Structure):
                 ("fc2_w", _fp), ("fc2_b", _fp)]
 
 
+class CsrGso(C.Structure):
+    """stgcn_csr_gso: a sparse graph shift operator, CSR device arrays of gso and of gso^T."""
+    _fields_ = [("N", C.c_int32), ("nnz", C.c_int32), ("row_ptr", _fp), ("col", _fp), ("val", _fp),
+                ("t_row_ptr", _fp), ("t_col", _fp), ("t_val", _fp)]
+
+
 # every symbol include/stgcn_b200.h declares: (name, restype, argtypes)
 _P = C.POINTER
 _sz = C.c_size_t
@@ -122,6 +128,18 @@ _SIGNATURES = [
     ("stgcn_stblock_infer", C.c_int, [_P(StblockDesc), _fp, _P(StblockParams), _fp, _fp, _sz, C.c_uint64, _fp]),
     ("stgcn_outblock_infer_sizes", C.c_int, [_P(OutblockDesc), _P(_sz)]),
     ("stgcn_outblock_infer", C.c_int, [_P(OutblockDesc), _fp, _P(OutblockParams), _fp, _fp, _sz, C.c_uint64, _fp]),
+    ("stgcn_gconv_sizes_csr", C.c_int, [_P(GconvDesc), _P(CsrGso), _P(_sz), _P(_sz)]),
+    ("stgcn_gconv_fwd_csr", C.c_int, [_P(GconvDesc), _fp, _P(GconvParams), _P(CsrGso), _fp, _fp, _fp, _sz, _fp]),
+    ("stgcn_gconv_bwd_csr", C.c_int, [_P(GconvDesc), _fp, _fp, _fp, _P(GconvParams), _P(CsrGso), _P(GconvGrads), _fp,
+                                      _fp, _sz, _fp]),
+    ("stgcn_stblock_sizes_csr", C.c_int, [_P(StblockDesc), _P(CsrGso), _P(_sz), _P(_sz)]),
+    ("stgcn_stblock_fwd_csr", C.c_int, [_P(StblockDesc), _fp, _P(StblockParams), _P(CsrGso), _fp, _fp, _fp, _sz,
+                                        C.c_uint64, _fp]),
+    ("stgcn_stblock_bwd_csr", C.c_int, [_P(StblockDesc), _fp, _fp, _fp, _P(StblockParams), _P(CsrGso), _P(StblockGrads),
+                                        _fp, _fp, _sz, C.c_uint64, _fp]),
+    ("stgcn_stblock_infer_sizes_csr", C.c_int, [_P(StblockDesc), _P(CsrGso), _P(_sz)]),
+    ("stgcn_stblock_infer_csr", C.c_int, [_P(StblockDesc), _fp, _P(StblockParams), _P(CsrGso), _fp, _fp, _sz,
+                                          C.c_uint64, _fp]),
     ("stgcn_eval_accumulate", C.c_int, [_fp, _fp, C.c_int32, C.c_int32, _fp, _fp, _fp, _fp]),
     ("stgcn_umma_selftest", C.c_int, [C.c_int, _fp, _fp, _fp, C.c_int, C.c_int, C.c_int, C.c_uint32, C.c_uint32,
                                       C.c_uint32, C.c_uint32, _fp]),

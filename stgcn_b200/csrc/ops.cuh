@@ -18,6 +18,7 @@
 #include "umma_x3.cuh"
 #include "umma_fb0.cuh"
 #include "umma_fb2.cuh"
+#include "spmm.cuh"
 
 namespace stgcn {
 namespace ops {
@@ -450,12 +451,22 @@ inline bool umma_linear(const simt::bf16* in, const simt::bf16* w_bf, const floa
 }
 
 // ============================ graph convolution layer ========================================
-// node contraction through tcgen05 (bf16, supported shapes) or the SIMT kernel
+// The graph shift operator of a graph conv is the dense (N, N) matrix of stgcn_gconv_params.gso, or -- when the
+// block-level and layer calls receive a `csr` operand (the *_csr entry points) -- a CSR operator, whose node contraction
+// runs on the SpMM kernel of spmm.cuh.  A CSR operand never takes the fused Chebyshev kernel (gconv_fused) nor reserves
+// the dense bf16 operator image: it runs the unfused recurrence with the node contraction swapped.
+inline spmm::Csr csr_dir(const stgcn_csr_gso& op, int trans) {
+  return trans ? spmm::Csr{op.N, op.t_row_ptr, op.t_col, op.t_val} : spmm::Csr{op.N, op.row_ptr, op.col, op.val};
+}
+
+// node contraction through the CSR SpMM (sparse operator), tcgen05 (bf16, supported shapes) or the SIMT kernel
 template <class T>
 struct GsoRunner {
   const float* M; int trans, N, C; long long G; cudaStream_t stream;
   const simt::bf16* mbf = nullptr;   // prepared bf16 operator (tcgen05 path) or nullptr
+  const stgcn_csr_gso* csr = nullptr;
   void operator()(const T* in, const T* aux, T* out, float alpha, float beta) const {
+    if (csr) { spmm::launch_spmm<T>(csr_dir(*csr, trans), in, aux, out, C, G, alpha, beta, stream); return; }
     if constexpr (std::is_same<T, simt::bf16>::value) {
       if (mbf) { umma::launch_gso_umma(mbf, in, aux, out, N, C, G, alpha, beta, stream); return; }
     }
@@ -466,8 +477,10 @@ struct GsoRunner {
 };
 template <class T>
 inline GsoRunner<T> make_gso_runner(const float* M, int trans, int N, int C, long long G, simt::bf16* mbf_buf,
-                                    cudaStream_t stream, cudaStream_t prep_stream) {
+                                    cudaStream_t stream, cudaStream_t prep_stream, const stgcn_csr_gso* csr = nullptr) {
   GsoRunner<T> r{M, trans, N, C, G, stream};
+  r.csr = csr;
+  if (csr) return r;
   if constexpr (std::is_same<T, simt::bf16>::value) {
     if (mbf_buf && umma::gso_supported(N, C, G)) {
       int Kp = (N + 63) / 64 * 64;
@@ -493,7 +506,8 @@ inline size_t gconv_saved_elems(const stgcn_gconv_desc& d) {
 }
 
 template <class T>
-inline bool gconv_fused(const stgcn_gconv_desc& d) {
+inline bool gconv_fused(const stgcn_gconv_desc& d, const stgcn_csr_gso* csr) {
+  if (csr) return false;
   if constexpr (std::is_same<T, simt::bf16>::value) {
     const int depth = gconv_stack_depth(d), taps = d.gconv == STGCN_GCONV_CHEB ? d.Ks : 1;
     return depth >= 2 && umma::cheb_supported(d.N, d.c_out, depth, taps, (long long)d.B * d.T);
@@ -505,21 +519,21 @@ inline bool gconv_fused(const stgcn_gconv_desc& d) {
 // planes == false (inference, fused kernel only): stack holds plane 0 alone; planes 1.. never reach HBM.
 template <class T>
 inline void gconv_fwd(const stgcn_gconv_desc& d, const T* x, const stgcn_gconv_params& p, T* y, T* stack, Ctx c,
-                      bool planes = true) {
+                      bool planes = true, const stgcn_csr_gso* csr = nullptr) {
   gconv_check(d);
   ScopedMark sm(c.ws);
   const long long rows = (long long)d.B * d.T * d.N;
   const int C = d.c_out;
   const size_t plane = (size_t)rows * C;
   float* wat = c.K().take<float>(d.c_in > C ? (size_t)d.c_in * C : 0);
-  simt::bf16* mbf = c.K().take<simt::bf16>(std::is_same<T, simt::bf16>::value ? umma::gso_prep_elems(d.N) : 0);
+  simt::bf16* mbf = c.K().take<simt::bf16>(std::is_same<T, simt::bf16>::value && !csr ? umma::gso_prep_elems(d.N) : 0);
   simt::bf16* wbf = c.K().take<simt::bf16>(std::is_same<T, simt::bf16>::value ? (size_t)d.c_in * C : 0);
   simt::bf16* wbf2 = c.K().take<simt::bf16>(std::is_same<T, simt::bf16>::value ? (size_t)(d.Ks > 1 ? d.Ks : 1) * C * C : 0);
   // fused Chebyshev / first-order kernel (umma_cheb.cuh): recurrence + weight GEMMs + bias/residual/ReLU in one pass
   const int fdepth = gconv_stack_depth(d), ftaps = d.gconv == STGCN_GCONV_CHEB ? d.Ks : 1;
-  const bool fused = gconv_fused<T>(d);
+  const bool fused = gconv_fused<T>(d, csr);
   if (c.dry()) return;
-  STGCN_CHECK(p.w && p.gso, STGCN_E_INVALID, "gconv: missing weight or gso");
+  STGCN_CHECK(p.w && (p.gso || csr), STGCN_E_INVALID, "gconv: missing weight or gso");
   STGCN_CHECK(planes || fused, STGCN_E_INVALID, "gconv_fwd: only the fused kernel runs without the stack planes");
   T* x0 = stack;
   bool align_done = false, mix_done = false;
@@ -557,7 +571,7 @@ inline void gconv_fwd(const stgcn_gconv_desc& d, const T* x, const stgcn_gconv_p
       return;
     }
   }
-  auto gso = make_gso_runner<T>(p.gso, 0, d.N, C, (long long)d.B * d.T, mbf, c.stream, c.ps());
+  auto gso = make_gso_runner<T>(p.gso, 0, d.N, C, (long long)d.B * d.T, mbf, c.stream, c.ps(), csr);
   c.prep_ready();
   TapArgs<T> t{};
   t.bias = p.b; t.out = y; t.rows = rows; t.Cin = C; t.Co = C; t.ldo = C;
@@ -596,7 +610,8 @@ inline void gconv_fwd(const stgcn_gconv_desc& d, const T* x, const stgcn_gconv_p
 
 template <class T>
 inline void gconv_bwd(const stgcn_gconv_desc& d, const T* x, const T* stack, const T* y, const T* dy,
-                      const stgcn_gconv_params& p, const stgcn_gconv_grads& gr, T* dx, Ctx c, T* dst_ext = nullptr) {
+                      const stgcn_gconv_params& p, const stgcn_gconv_grads& gr, T* dx, Ctx c, T* dst_ext = nullptr,
+                      const stgcn_csr_gso* csr = nullptr) {
   // dst_ext: optional caller-owned [depth][rows, c_out] buffer for the stack gradients; plane 0 (the gradient w.r.t. the
   // aligned input) then outlives this call, and with dx == nullptr the caller applies the align conv's data gradient
   // itself (stblock_bwd: fused into the first temporal conv's backward, umma_fb0.cuh)
@@ -612,12 +627,12 @@ inline void gconv_bwd(const stgcn_gconv_desc& d, const T* x, const T* stack, con
   float* wT = c.K().take<float>((size_t)ntw * C * C);
   float* dwt = c.K().take<float>((size_t)(ntw * C + 1) * C);
   float* dwa = c.K().take<float>(d.c_in > C ? (size_t)(d.c_in + 1) * C : 0);
-  simt::bf16* mbf = c.K().take<simt::bf16>(std::is_same<T, simt::bf16>::value ? umma::gso_prep_elems(d.N) : 0);
+  simt::bf16* mbf = c.K().take<simt::bf16>(std::is_same<T, simt::bf16>::value && !csr ? umma::gso_prep_elems(d.N) : 0);
   float* part = c.KW().take<float>(std::max(wgrad_partial_elems(rows, ntw * C + 1, C),
                                           d.c_in > C ? wgrad_partial_elems(rows, d.c_in + 1, C) : (size_t)0));
   simt::bf16* wbf = c.K().take<simt::bf16>(std::is_same<T, simt::bf16>::value ? (size_t)ntw * C * C : 0);       // stack-gradient weights
   simt::bf16* wbfa = c.K().take<simt::bf16>(std::is_same<T, simt::bf16>::value ? (size_t)d.c_in * C : 0);      // align data-gradient weights
-  const bool fused = gconv_fused<T>(d);
+  const bool fused = gconv_fused<T>(d, csr);
   if (c.dry()) return;
   if constexpr (std::is_same<T, simt::bf16>::value) {
     if (fused) {
@@ -637,7 +652,8 @@ inline void gconv_bwd(const stgcn_gconv_desc& d, const T* x, const T* stack, con
   if (!fused)
     STGCN_LAUNCH(relu_bwd_kernel<T>, ceil_div(ceil_div(plane, 8), 256), 256, 0, c.stream, dy, y, dg, (long long)plane, d.relu);
 
-  auto gso = make_gso_runner<T>(p.gso, 1, d.N, C, (long long)d.B * d.T, fused ? nullptr : mbf, c.stream, c.ps());
+  // the adjoint recurrence contracts with gso^T: the dense path reads M transposed, a CSR operand its transpose arrays
+  auto gso = make_gso_runner<T>(p.gso, 1, d.N, C, (long long)d.B * d.T, fused ? nullptr : mbf, c.stream, c.ps(), csr);
   TapArgs<T> t{};
   t.in = dg; t.bias = nullptr; t.rows = rows; t.Cin = C; t.Co = C; t.ntaps = 1; t.ldo = C;
   t.map = RowMap{d.T, d.T, d.N, 0, 0};
@@ -948,12 +964,12 @@ inline StSaved<T> st_saved(const stgcn_stblock_desc& d, const StGeom& g, Arena& 
 
 template <class T>
 inline void stblock_fwd(const stgcn_stblock_desc& d, const T* x, const stgcn_stblock_params& p, T* y,
-                        Arena& sv, Ctx c, uint64_t seed) {
+                        Arena& sv, Ctx c, uint64_t seed, const stgcn_csr_gso* csr = nullptr) {
   StGeom g = st_geom(d);
   StSaved<T> s = st_saved<T>(d, g, sv);
   const bool first = d.c_in == 1;   // label only: distinguishes the two blocks of the default model in profiles
   { Tag t(first ? "st0.tc1.fwd" : "st1.tc1.fwd"); tconv_fwd<T>(g.tc1, x, p.tc1, s.h1, s.z1, c, tconv_qonly<T>(g.tc1)); }
-  { Tag t(first ? "st0.gc.fwd" : "st1.gc.fwd"); gconv_fwd<T>(g.gc, s.h1, p.gc, s.h2, s.stack, c); }
+  { Tag t(first ? "st0.gc.fwd" : "st1.gc.fwd"); gconv_fwd<T>(g.gc, s.h1, p.gc, s.h2, s.stack, c, true, csr); }
   { Tag t(first ? "st0.tc2.fwd" : "st1.tc2.fwd"); tconv_fwd<T>(g.tc2, s.h2, p.tc2, s.h3, s.z2, c, tconv_qonly<T>(g.tc2)); }
   { Tag t(first ? "st0.ln.fwd" : "st1.ln.fwd"); lnorm_fwd<T>(g.ln, s.h3, p.ln_w, p.ln_b, y, s.stats, seed, c.stream, c.dry()); }
 }
@@ -963,7 +979,7 @@ inline void stblock_fwd(const stgcn_stblock_desc& d, const T* x, const stgcn_stb
 // the pre-activations / recurrence planes that only a backward reads are not stored where the kernel can skip them.
 template <class T>
 inline void stblock_infer(const stgcn_stblock_desc& d, const T* x, const stgcn_stblock_params& p, T* y, Ctx c,
-                          uint64_t seed) {
+                          uint64_t seed, const stgcn_csr_gso* csr = nullptr) {
   StGeom g = st_geom(d);
   const bool first = d.c_in == 1;
   const bool q1 = tconv_qonly<T>(g.tc1), q2 = tconv_qonly<T>(g.tc2);
@@ -978,10 +994,10 @@ inline void stblock_infer(const stgcn_stblock_desc& d, const T* x, const stgcn_s
       Tag t(first ? "st0.tc1.infer" : "st1.tc1.infer");
       tconv_fwd<T>(g.tc1, x, p.tc1, h1, z1, c, q1);
     }
-    const bool planes = !gconv_fused<T>(g.gc);
+    const bool planes = !gconv_fused<T>(g.gc, csr);
     T* stack = c.ws.take<T>(planes ? gconv_saved_elems(g.gc) : (size_t)g.rows1 * d.c2);
     Tag t(first ? "st0.gc.infer" : "st1.gc.infer");
-    gconv_fwd<T>(g.gc, h1, p.gc, h2, stack, c, planes);
+    gconv_fwd<T>(g.gc, h1, p.gc, h2, stack, c, planes, csr);
   }
   T* h3 = c.ws.take<T>((size_t)g.rows2 * d.c3);
   {
@@ -997,7 +1013,8 @@ inline void stblock_infer(const stgcn_stblock_desc& d, const T* x, const stgcn_s
 
 template <class T>
 inline void stblock_bwd(const stgcn_stblock_desc& d, const T* x, Arena& sv, const T* dy,
-                        const stgcn_stblock_params& p, const stgcn_stblock_grads& gr, T* dx, Ctx c, uint64_t seed) {
+                        const stgcn_stblock_params& p, const stgcn_stblock_grads& gr, T* dx, Ctx c, uint64_t seed,
+                        const stgcn_csr_gso* csr = nullptr) {
   StGeom g = st_geom(d);
   StSaved<T> s = st_saved<T>(d, g, sv);
   ScopedMark sm(c.ws);
@@ -1068,7 +1085,7 @@ inline void stblock_bwd(const stgcn_stblock_desc& d, const T* x, Arena& sv, cons
   T* dz1 = c.KW().take<T>(fbg_shape ? (size_t)g.rows1 * 2 * d.c1 : 0);
   const bool fbg = fbg_shape && !c.dry();
   { Tag t(first ? "st0.gc.bwd" : "st1.gc.bwd"); gconv_bwd<T>(g.gc, s.h1, s.stack, s.h2, dh2, p.gc, gr.gc, (fb0 || fbg) ? nullptr : dh1, c,
-                                                               fb0_shape ? dst_ext : (fbg_shape ? dst_ext2 : nullptr)); }
+                                                               fb0_shape ? dst_ext : (fbg_shape ? dst_ext2 : nullptr), csr); }
   if (fb0) {
     if constexpr (std::is_same<T, simt::bf16>::value) {
       Tag t("st0.tc1.bwd");

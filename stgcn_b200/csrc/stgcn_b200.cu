@@ -35,6 +35,16 @@ using bf16 = __nv_bfloat16;
   } while (0)
 inline size_t elem_size(int precision) { return precision == STGCN_PREC_BF16 ? sizeof(bf16) : sizeof(float); }
 inline size_t max2(size_t a, size_t b) { return a > b ? a : b; }
+// argument checks of the *_csr entry points: the CSR operand replaces the dense one, so the dense pointer must be NULL
+inline void check_csr(const stgcn_csr_gso* op, int32_t N, const float* dense_gso) {
+  STGCN_CHECK(op, STGCN_E_INVALID, "null CSR operator");
+  STGCN_CHECK(!dense_gso, STGCN_E_INVALID, "a CSR operator call takes no dense gso");
+  STGCN_CHECK(op->N == N, STGCN_E_INVALID, "CSR operator size differs from the desc's N");
+  STGCN_CHECK(op->nnz >= 0, STGCN_E_INVALID, "CSR operator with negative nnz");
+  STGCN_CHECK(op->row_ptr && op->t_row_ptr, STGCN_E_INVALID, "CSR operator without row offsets");
+  STGCN_CHECK(op->nnz == 0 || (op->col && op->val && op->t_col && op->t_val), STGCN_E_INVALID,
+              "CSR operator without column / value arrays");
+}
 
 // Block-level calls (stblock / outblock).  The workspace is split into a "keep" region -- prepared weights and gradient
 // accumulators, which helper-stream work reads and writes asynchronously and which therefore live for the whole call
@@ -337,6 +347,117 @@ int stgcn_outblock_infer(const stgcn_outblock_desc* d, const void* x, const stgc
     STGCN_CHECK(d && p && x && y && workspace, STGCN_E_INVALID, "null argument");
     STGCN_DISPATCH(d->precision, run_block(workspace, workspace_bytes, as_stream(stream), [&](ops::Ctx c) {
                      ops::outblock_infer<T>(*d, (const T*)x, *p, (float*)y, c, dropout_seed);
+                   }));
+  });
+}
+
+// ---------------------------------------------------------------- sparse graph shift operators
+// The dense entry points above with a CSR operand: same layouts, buffers and launch order, the node contraction on the
+// SpMM kernel (spmm.cuh).  Shapes alone decide every allocation, so the size queries need only op->N.
+int stgcn_gconv_sizes_csr(const stgcn_gconv_desc* d, const stgcn_csr_gso* op, size_t* saved_bytes,
+                          size_t* workspace_bytes) {
+  return guarded([&] {
+    STGCN_CHECK(d, STGCN_E_INVALID, "null desc");
+    check_csr(op, d->N, nullptr);
+    Arena ws(nullptr, 0);
+    ops::Ctx c{ws, nullptr};
+    stgcn_gconv_params p{};
+    stgcn_gconv_grads g{};
+    Arena sv(nullptr, 0);
+    STGCN_DISPATCH(d->precision, ops::gconv_fwd<T>(*d, nullptr, p, nullptr, nullptr, c, true, op);
+                   ops::gconv_bwd<T>(*d, nullptr, nullptr, nullptr, nullptr, p, g, nullptr, c, nullptr, op);
+                   sv.take<T>(ops::gconv_saved_elems(*d)); sv.take<T>((size_t)d->B * d->T * d->N * d->c_out));
+    if (saved_bytes) *saved_bytes = sv.peak;
+    if (workspace_bytes) *workspace_bytes = ws.peak;
+  });
+}
+int stgcn_gconv_fwd_csr(const stgcn_gconv_desc* d, const void* x, const stgcn_gconv_params* p, const stgcn_csr_gso* op,
+                        void* y, void* saved, void* workspace, size_t workspace_bytes, void* stream) {
+  return guarded([&] {
+    STGCN_CHECK(d && p && x && y && saved && workspace, STGCN_E_INVALID, "null argument");
+    check_csr(op, d->N, p->gso);
+    Arena ws(workspace, workspace_bytes);
+    Arena sv(saved, (size_t)-1);
+    size_t ny = (size_t)d->B * d->T * d->N * d->c_out;
+    STGCN_DISPATCH(d->precision, T* stack = sv.take<T>(ops::gconv_saved_elems(*d)); T* ycopy = sv.take<T>(ny);
+                   ops::gconv_fwd<T>(*d, (const T*)x, *p, (T*)y, stack, ops::Ctx{ws, as_stream(stream)}, true, op);
+                   ops::copy<T>(ycopy, (const T*)y, ny, as_stream(stream)));
+  });
+}
+int stgcn_gconv_bwd_csr(const stgcn_gconv_desc* d, const void* x, const void* saved, const void* dy,
+                        const stgcn_gconv_params* p, const stgcn_csr_gso* op, const stgcn_gconv_grads* g, void* dx,
+                        void* workspace, size_t workspace_bytes, void* stream) {
+  return guarded([&] {
+    STGCN_CHECK(d && p && g && x && saved && dy && workspace, STGCN_E_INVALID, "null argument");
+    check_csr(op, d->N, p->gso);
+    Arena ws(workspace, workspace_bytes);
+    Arena sv(const_cast<void*>(saved), (size_t)-1);
+    STGCN_DISPATCH(d->precision, T* stack = sv.take<T>(ops::gconv_saved_elems(*d));
+                   T* ycopy = sv.take<T>((size_t)d->B * d->T * d->N * d->c_out);
+                   ops::gconv_bwd<T>(*d, (const T*)x, stack, ycopy, (const T*)dy, *p, *g, (T*)dx,
+                                     ops::Ctx{ws, as_stream(stream)}, nullptr, op));
+  });
+}
+int stgcn_stblock_sizes_csr(const stgcn_stblock_desc* d, const stgcn_csr_gso* op, size_t* saved_bytes,
+                            size_t* workspace_bytes) {
+  return guarded([&] {
+    STGCN_CHECK(d, STGCN_E_INVALID, "null desc");
+    check_csr(op, d->N, nullptr);
+    Arena ws(nullptr, 0), sv(nullptr, 0), sv2(nullptr, 0), keep_f(nullptr, 0), keep_b(nullptr, 0);
+    ops::Ctx cf{ws, nullptr}, cb{ws, nullptr};
+    cf.keep = &keep_f; cb.keep = &keep_b;
+    stgcn_stblock_params p{};
+    stgcn_stblock_grads g{};
+    STGCN_DISPATCH(d->precision, ops::stblock_fwd<T>(*d, nullptr, p, nullptr, sv, cf, 0, op);
+                   ops::stblock_bwd<T>(*d, nullptr, sv2, nullptr, p, g, nullptr, cb, 0, op));
+    if (saved_bytes) *saved_bytes = max2(sv.peak, 256);
+    if (workspace_bytes) *workspace_bytes = max2(ws.peak, 256) + Arena::align_up(max2(keep_f.peak, keep_b.peak));
+  });
+}
+int stgcn_stblock_fwd_csr(const stgcn_stblock_desc* d, const void* x, const stgcn_stblock_params* p,
+                          const stgcn_csr_gso* op, void* y, void* saved, void* workspace, size_t workspace_bytes,
+                          uint64_t dropout_seed, void* stream) {
+  return guarded([&] {
+    STGCN_CHECK(d && p && x && y && saved && workspace, STGCN_E_INVALID, "null argument");
+    check_csr(op, d->N, p->gc.gso);
+    STGCN_DISPATCH(d->precision, run_block(workspace, workspace_bytes, as_stream(stream), [&](ops::Ctx c) {
+                     Arena sv(c.dry() ? nullptr : saved, (size_t)-1);
+                     ops::stblock_fwd<T>(*d, (const T*)x, *p, (T*)y, sv, c, dropout_seed, op);
+                   }));
+  });
+}
+int stgcn_stblock_bwd_csr(const stgcn_stblock_desc* d, const void* x, const void* saved, const void* dy,
+                          const stgcn_stblock_params* p, const stgcn_csr_gso* op, const stgcn_stblock_grads* g,
+                          void* dx, void* workspace, size_t workspace_bytes, uint64_t dropout_seed, void* stream) {
+  return guarded([&] {
+    STGCN_CHECK(d && p && g && x && saved && dy && workspace, STGCN_E_INVALID, "null argument");
+    check_csr(op, d->N, p->gc.gso);
+    STGCN_DISPATCH(d->precision, run_block(workspace, workspace_bytes, as_stream(stream), [&](ops::Ctx c) {
+                     Arena sv(c.dry() ? nullptr : const_cast<void*>(saved), (size_t)-1);
+                     ops::stblock_bwd<T>(*d, (const T*)x, sv, (const T*)dy, *p, *g, (T*)dx, c, dropout_seed, op);
+                   }));
+  });
+}
+int stgcn_stblock_infer_sizes_csr(const stgcn_stblock_desc* d, const stgcn_csr_gso* op, size_t* workspace_bytes) {
+  return guarded([&] {
+    STGCN_CHECK(d, STGCN_E_INVALID, "null desc");
+    check_csr(op, d->N, nullptr);
+    Arena ws(nullptr, 0), keep(nullptr, 0);
+    ops::Ctx c{ws, nullptr};
+    c.keep = &keep;
+    stgcn_stblock_params p{};
+    STGCN_DISPATCH(d->precision, ops::stblock_infer<T>(*d, nullptr, p, nullptr, c, 0, op));
+    if (workspace_bytes) *workspace_bytes = max2(ws.peak, 256) + Arena::align_up(keep.peak);
+  });
+}
+int stgcn_stblock_infer_csr(const stgcn_stblock_desc* d, const void* x, const stgcn_stblock_params* p,
+                            const stgcn_csr_gso* op, void* y, void* workspace, size_t workspace_bytes,
+                            uint64_t dropout_seed, void* stream) {
+  return guarded([&] {
+    STGCN_CHECK(d && p && x && y && workspace, STGCN_E_INVALID, "null argument");
+    check_csr(op, d->N, p->gc.gso);
+    STGCN_DISPATCH(d->precision, run_block(workspace, workspace_bytes, as_stream(stream), [&](ops::Ctx c) {
+                     ops::stblock_infer<T>(*d, (const T*)x, *p, (T*)y, c, dropout_seed, op);
                    }));
   });
 }

@@ -29,6 +29,7 @@ import torch.nn as nn
 from . import _lib as L
 from . import layers
 from .data import DeviceWindows
+from .gso import CsrOperator
 
 __all__ = ["eval_accumulate", "evaluate_model", "evaluate_metric", "WindowEvaluator"]
 
@@ -129,7 +130,13 @@ class WindowEvaluator:
 
     def _addresses(self):
         """Addresses of every tensor the captured forward reads from the model."""
-        gsos = [m.gso for m in self.model.modules() if torch.is_tensor(getattr(m, "gso", None))]
+        gsos = []
+        for m in self.model.modules():
+            g = getattr(m, "gso", None)
+            if torch.is_tensor(g):
+                gsos.append(g)
+            elif isinstance(g, CsrOperator):           # the CSR arrays the sparse path reads
+                gsos.extend(g.tensors())
         return tuple(t.data_ptr() for t in (*self.model.parameters(), *gsos))
 
     def _capture(self):

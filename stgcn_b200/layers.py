@@ -28,6 +28,7 @@ import torch.nn as nn
 import torch.nn.init as init
 
 from . import _lib as L
+from . import gso as G
 
 __all__ = ["Align", "CausalConv1d", "CausalConv2d", "TemporalConvLayer", "ChebGraphConv", "GraphConv",
            "GraphConvLayer", "STConvBlock", "OutputBlock", "set_precision", "get_precision"]
@@ -127,10 +128,23 @@ def _f32c(t: Optional[torch.Tensor]) -> Optional[torch.Tensor]:
     return t.contiguous()
 
 
-def _sizes(fn, desc) -> Tuple[int, int]:
+def _sizes(fn, desc, op: Optional[G.CsrOperator] = None) -> Tuple[int, int]:
+    """(saved, workspace) bytes from a *_sizes entry point, or from its *_csr twin when a sparse operator is given."""
     sv, ws = C.c_size_t(0), C.c_size_t(0)
-    L.check(fn(C.byref(desc), C.byref(sv), C.byref(ws)))
+    if op is None:
+        L.check(fn(C.byref(desc), C.byref(sv), C.byref(ws)))
+    else:
+        L.check(fn(C.byref(desc), C.byref(op.c_struct()), C.byref(sv), C.byref(ws)))
     return int(sv.value), int(ws.value)
+
+
+def _sparse(gso) -> Optional[G.CsrOperator]:
+    """The CSR operator when ``gso`` takes the sparse path (the *_csr entry points), else None (dense gso pointer)."""
+    return gso if isinstance(gso, G.CsrOperator) else None
+
+
+def _dense_ptr(gso) -> Optional[int]:
+    return None if isinstance(gso, G.CsrOperator) else _ptr(gso)
 
 
 def _grad_like(p: Optional[torch.Tensor], needed: bool) -> Optional[torch.Tensor]:
@@ -194,17 +208,22 @@ class _GconvFn(torch.autograd.Function):
         B, T, N, c_in, c_out, Ks, gconv, relu, residual = dims
         lib = L.lib()
         desc = L.GconvDesc(B, T, N, c_in, c_out, Ks, gconv, relu, residual, L.PREC[_PRECISION])
-        sv_bytes, ws_bytes = _sizes(lib.stgcn_gconv_sizes, desc)
+        op = _sparse(gso)
+        sv_bytes, ws_bytes = _sizes(lib.stgcn_gconv_sizes_csr if op else lib.stgcn_gconv_sizes, desc, op)
         dev = x_cl.device
         saved = torch.empty(sv_bytes, dtype=torch.uint8, device=dev)
         ws = _workspace(dev, ws_bytes)
         y = torch.empty((B, T, N, c_out), dtype=x_cl.dtype, device=dev)
-        params = L.GconvParams(_ptr(align_w), _ptr(align_b), _ptr(w), _ptr(b), _ptr(gso))
+        params = L.GconvParams(_ptr(align_w), _ptr(align_b), _ptr(w), _ptr(b), _dense_ptr(gso))
         with torch.cuda.device(dev):      # kernels, helper streams and events follow the CUDA current device
-            L.check(lib.stgcn_gconv_fwd(C.byref(desc), x_cl.data_ptr(), C.byref(params), y.data_ptr(), saved.data_ptr(),
-                                        ws.data_ptr(), ws.numel(), _stream(dev)))
-        ctx.desc = desc
-        ctx.save_for_backward(x_cl, saved, gso, align_w, align_b, w, b)
+            if op is None:
+                L.check(lib.stgcn_gconv_fwd(C.byref(desc), x_cl.data_ptr(), C.byref(params), y.data_ptr(),
+                                            saved.data_ptr(), ws.data_ptr(), ws.numel(), _stream(dev)))
+            else:
+                L.check(lib.stgcn_gconv_fwd_csr(C.byref(desc), x_cl.data_ptr(), C.byref(params), C.byref(op.c_struct()),
+                                                y.data_ptr(), saved.data_ptr(), ws.data_ptr(), ws.numel(), _stream(dev)))
+        ctx.desc, ctx.op = desc, op
+        ctx.save_for_backward(x_cl, saved, None if op else gso, align_w, align_b, w, b)
         return y
 
     @staticmethod
@@ -215,14 +234,21 @@ class _GconvFn(torch.autograd.Function):
         need = ctx.needs_input_grad
         dx = torch.empty_like(x_cl) if need[0] else None
         g = [_grad_like(align_w, need[3]), _grad_like(align_b, need[4]), _grad_like(w, need[5]), _grad_like(b, need[6])]
-        _, ws_bytes = _sizes(lib.stgcn_gconv_sizes, ctx.desc)
+        op = ctx.op
+        _, ws_bytes = _sizes(lib.stgcn_gconv_sizes_csr if op else lib.stgcn_gconv_sizes, ctx.desc, op)
         ws = _workspace(dev, ws_bytes)
         params = L.GconvParams(_ptr(align_w), _ptr(align_b), _ptr(w), _ptr(b), _ptr(gso))
         grads = L.GconvGrads(*[_ptr(t) for t in g])
         dy = dy.to(x_cl.dtype).contiguous()
         with torch.cuda.device(dev):      # kernels, helper streams and events follow the CUDA current device
-            L.check(lib.stgcn_gconv_bwd(C.byref(ctx.desc), x_cl.data_ptr(), saved.data_ptr(), dy.data_ptr(),
-                                        C.byref(params), C.byref(grads), _ptr(dx), ws.data_ptr(), ws.numel(), _stream(dev)))
+            if op is None:
+                L.check(lib.stgcn_gconv_bwd(C.byref(ctx.desc), x_cl.data_ptr(), saved.data_ptr(), dy.data_ptr(),
+                                            C.byref(params), C.byref(grads), _ptr(dx), ws.data_ptr(), ws.numel(),
+                                            _stream(dev)))
+            else:
+                L.check(lib.stgcn_gconv_bwd_csr(C.byref(ctx.desc), x_cl.data_ptr(), saved.data_ptr(), dy.data_ptr(),
+                                                C.byref(params), C.byref(op.c_struct()), C.byref(grads), _ptr(dx),
+                                                ws.data_ptr(), ws.numel(), _stream(dev)))
         return (dx, None, None, *g)
 
 
@@ -277,7 +303,8 @@ class _STBlockFn(torch.autograd.Function):
         lib = L.lib()
         desc = L.StblockDesc(B, T, N, c_in, c1, c2, c3, Kt, Ks, act, gconv, int(training), float(p_drop), float(eps),
                              L.PREC[_PRECISION])
-        sv_bytes, ws_bytes = _sizes(lib.stgcn_stblock_sizes, desc)
+        op = _sparse(gso)
+        sv_bytes, ws_bytes = _sizes(lib.stgcn_stblock_sizes_csr if op else lib.stgcn_stblock_sizes, desc, op)
         dev = x_cl.device
         saved = torch.empty(sv_bytes, dtype=torch.uint8, device=dev)
         ws = _workspace(dev, ws_bytes)
@@ -285,17 +312,22 @@ class _STBlockFn(torch.autograd.Function):
         seed = _next_seed() if (training and p_drop > 0) else 0
         cparams = _STBlockFn._pack(params, gso)
         with torch.cuda.device(dev):      # kernels, helper streams and events follow the CUDA current device
-            L.check(lib.stgcn_stblock_fwd(C.byref(desc), x_cl.data_ptr(), C.byref(cparams), y.data_ptr(), saved.data_ptr(),
-                                          ws.data_ptr(), ws.numel(), seed, _stream(dev)))
-        ctx.desc, ctx.seed, ctx.ws_bytes = desc, seed, ws_bytes
-        ctx.save_for_backward(x_cl, saved, gso, *params)
+            if op is None:
+                L.check(lib.stgcn_stblock_fwd(C.byref(desc), x_cl.data_ptr(), C.byref(cparams), y.data_ptr(),
+                                              saved.data_ptr(), ws.data_ptr(), ws.numel(), seed, _stream(dev)))
+            else:
+                L.check(lib.stgcn_stblock_fwd_csr(C.byref(desc), x_cl.data_ptr(), C.byref(cparams),
+                                                  C.byref(op.c_struct()), y.data_ptr(), saved.data_ptr(), ws.data_ptr(),
+                                                  ws.numel(), seed, _stream(dev)))
+        ctx.desc, ctx.seed, ctx.ws_bytes, ctx.op = desc, seed, ws_bytes, op
+        ctx.save_for_backward(x_cl, saved, None if op else gso, *params)
         return y
 
     @staticmethod
     def _pack(p, gso):
         (t1w, t1b, t1aw, t1ab, gaw, gab, gw, gb, t2w, t2b, t2aw, t2ab, lw, lb) = p
         return L.StblockParams(L.TconvParams(_ptr(t1w), _ptr(t1b), _ptr(t1aw), _ptr(t1ab)),
-                               L.GconvParams(_ptr(gaw), _ptr(gab), _ptr(gw), _ptr(gb), _ptr(gso)),
+                               L.GconvParams(_ptr(gaw), _ptr(gab), _ptr(gw), _ptr(gb), _dense_ptr(gso)),
                                L.TconvParams(_ptr(t2w), _ptr(t2b), _ptr(t2aw), _ptr(t2ab)), _ptr(lw), _ptr(lb))
 
     @staticmethod
@@ -309,12 +341,18 @@ class _STBlockFn(torch.autograd.Function):
         ws = _workspace(dev, ctx.ws_bytes)
         gp = [_ptr(t) for t in g]
         grads = L.StblockGrads(L.TconvGrads(*gp[0:4]), L.GconvGrads(*gp[4:8]), L.TconvGrads(*gp[8:12]), gp[12], gp[13])
+        op = ctx.op
         cparams = _STBlockFn._pack(params, gso)
         dy = dy.to(x_cl.dtype).contiguous()
         with torch.cuda.device(dev):      # kernels, helper streams and events follow the CUDA current device
-            L.check(lib.stgcn_stblock_bwd(C.byref(ctx.desc), x_cl.data_ptr(), saved.data_ptr(), dy.data_ptr(),
-                                          C.byref(cparams), C.byref(grads), _ptr(dx), ws.data_ptr(), ws.numel(), ctx.seed,
-                                          _stream(dev)))
+            if op is None:
+                L.check(lib.stgcn_stblock_bwd(C.byref(ctx.desc), x_cl.data_ptr(), saved.data_ptr(), dy.data_ptr(),
+                                              C.byref(cparams), C.byref(grads), _ptr(dx), ws.data_ptr(), ws.numel(),
+                                              ctx.seed, _stream(dev)))
+            else:
+                L.check(lib.stgcn_stblock_bwd_csr(C.byref(ctx.desc), x_cl.data_ptr(), saved.data_ptr(), dy.data_ptr(),
+                                                  C.byref(cparams), C.byref(op.c_struct()), C.byref(grads), _ptr(dx),
+                                                  ws.data_ptr(), ws.numel(), ctx.seed, _stream(dev)))
         return (dx, None, None, *g)
 
 
@@ -386,15 +424,23 @@ def _stblock_infer(x_cl, dims, gso, params):
     desc = L.StblockDesc(B, T, N, c_in, c1, c2, c3, Kt, Ks, act, gconv, int(training), float(p_drop), float(eps),
                          L.PREC[_PRECISION])
     ws_bytes = C.c_size_t(0)
-    L.check(lib.stgcn_stblock_infer_sizes(C.byref(desc), C.byref(ws_bytes)))
+    op = _sparse(gso)
+    if op is None:
+        L.check(lib.stgcn_stblock_infer_sizes(C.byref(desc), C.byref(ws_bytes)))
+    else:
+        L.check(lib.stgcn_stblock_infer_sizes_csr(C.byref(desc), C.byref(op.c_struct()), C.byref(ws_bytes)))
     dev = x_cl.device
     ws = _workspace(dev, int(ws_bytes.value))
     y = torch.empty((B, T - 2 * (Kt - 1), N, c3), dtype=x_cl.dtype, device=dev)
     seed = _next_seed() if (training and p_drop > 0) else 0
     cparams = _STBlockFn._pack(params, gso)
     with torch.cuda.device(dev):      # kernels, helper streams and events follow the CUDA current device
-        L.check(lib.stgcn_stblock_infer(C.byref(desc), x_cl.data_ptr(), C.byref(cparams), y.data_ptr(), ws.data_ptr(),
-                                        ws.numel(), seed, _stream(dev)))
+        if op is None:
+            L.check(lib.stgcn_stblock_infer(C.byref(desc), x_cl.data_ptr(), C.byref(cparams), y.data_ptr(),
+                                            ws.data_ptr(), ws.numel(), seed, _stream(dev)))
+        else:
+            L.check(lib.stgcn_stblock_infer_csr(C.byref(desc), x_cl.data_ptr(), C.byref(cparams), C.byref(op.c_struct()),
+                                                y.data_ptr(), ws.data_ptr(), ws.numel(), seed, _stream(dev)))
     return y
 
 
@@ -524,9 +570,17 @@ def _reset_graph_params(weight, bias):
         init.uniform_(bias, -bound, bound)
 
 
-def _gso_device(gso: torch.Tensor, like: torch.Tensor) -> torch.Tensor:
+def _gso_device(gso, like: torch.Tensor):
+    """The operator a forward on ``like`` (B, C, T, N) uses: a dense tensor on its device, or -- for a CsrOperator, a
+    torch sparse tensor or a scipy sparse matrix -- a CsrOperator there (converted once; the caller keeps the result)."""
+    if G.is_sparse_operator(gso):
+        op = G.as_operator(gso, like.device)
+        if op.N != like.shape[-1]:
+            raise ValueError(f"gso: a ({op.N}, {op.N}) operator for an input with {like.shape[-1]} vertices")
+        return op
     if not torch.is_tensor(gso):
-        raise TypeError("gso must be a dense torch tensor (N, N)")
+        raise TypeError("gso must be a dense torch tensor (N, N) or a sparse operator (stgcn_b200.gso.CsrOperator, "
+                        "a torch sparse COO / CSR tensor or a scipy sparse matrix)")
     if gso.device != like.device or gso.dtype != torch.float32 or not gso.is_contiguous():
         gso = gso.to(device=like.device, dtype=torch.float32).contiguous()
     return gso
@@ -534,7 +588,9 @@ def _gso_device(gso: torch.Tensor, like: torch.Tensor) -> torch.Tensor:
 
 class ChebGraphConv(nn.Module):
     """Chebyshev graph convolution (layers.py:122-172): x (B,C,T,N) -> (B,T,N,C_out).  ``gso`` is a plain
-    attribute (not a buffer), exactly as in the reference, so it stays out of the state_dict."""
+    attribute (not a buffer), exactly as in the reference, so it stays out of the state_dict.  A dense tensor takes the
+    dense path; a stgcn_b200.gso.CsrOperator, torch sparse tensor or scipy sparse matrix the CSR path (this holds for
+    every layer that takes ``gso``)."""
 
     def __init__(self, c_in, c_out, Ks, gso, bias):
         super().__init__()
@@ -641,6 +697,8 @@ class STConvBlock(nn.Module):
 
     def __init__(self, Kt, Ks, n_vertex, last_block_channel, channels, act_func, graph_conv_type, gso, bias, droprate):
         super().__init__()
+        if G.is_sparse_operator(gso) and tuple(gso.shape) != (n_vertex, n_vertex):
+            raise ValueError(f"STConvBlock: a {tuple(gso.shape)} sparse gso for n_vertex = {n_vertex}")
         self.tmp_conv1 = TemporalConvLayer(Kt, last_block_channel, channels[0], n_vertex, act_func)
         self.graph_conv = GraphConvLayer(graph_conv_type, channels[0], channels[1], Ks, gso, bias)
         self.tmp_conv2 = TemporalConvLayer(Kt, channels[1], channels[2], n_vertex, act_func)

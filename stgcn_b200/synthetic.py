@@ -1,10 +1,35 @@
 """Synthetic inputs of the BASELINE.json workloads that do not come from a dataset (no network, no dataset files on
-the GPU box): the seeded dense operator of the N=2048 roofline sweep (SURVEY.md §8d) and default-initialised models."""
+the GPU box): the seeded dense operator of the N=2048 roofline sweep (SURVEY.md §8d), seeded sparse k-nearest-neighbour
+operators for the CSR path, and default-initialised models."""
 from __future__ import annotations
 
 from types import SimpleNamespace
 
 import torch
+
+
+def knn_operator(n: int, degree: int, seed: int = 0, symmetric: bool = True):
+    """Seeded sparse graph shift operator of a k-nearest-neighbour graph, as a scipy CSR float32 matrix: n points
+    uniform in the unit square, each joined to its ``degree`` nearest others with Gaussian weights exp(-d^2 / s^2)
+    (s = the median neighbour distance).  symmetric: the union graph, D^-1/2 A D^-1/2 (the reference's sym_norm_adj,
+    utility.py:21-31), spectrum in [-1, 1]; else the directed graph, D^-1 A (rw_norm_adj, utility.py:33-42)."""
+    import numpy as np
+    import scipy.sparse as sp
+    from scipy.spatial import cKDTree
+    rng = np.random.default_rng(seed)
+    pts = rng.random((n, 2))
+    dist, idx = cKDTree(pts).query(pts, k=degree + 1)
+    dist, idx = dist[:, 1:], idx[:, 1:]                        # drop the point itself
+    scale = np.median(dist) or 1.0
+    w = np.exp(-(dist / scale) ** 2)
+    a = sp.csr_matrix((w.reshape(-1), (np.repeat(np.arange(n), degree), idx.reshape(-1))), shape=(n, n))
+    if symmetric:
+        a = a.maximum(a.T)
+        d = np.asarray(a.sum(axis=1)).reshape(-1) ** -0.5
+        a = sp.diags(d) @ a @ sp.diags(d)
+    else:
+        a = sp.diags(1.0 / np.asarray(a.sum(axis=1)).reshape(-1)) @ a
+    return sp.csr_matrix(a, dtype=np.float32)
 
 
 def synthetic_operator(n: int, seed: int = 0, dtype=torch.float32) -> torch.Tensor:
